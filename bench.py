@@ -86,6 +86,23 @@ def c3_data_bin(solids: int, wait_s: float = 600.0) -> str:
     return path
 
 
+DUMP_BYTES = 48 << 20   # bound on --dump-outputs' arrays (frames + pixel positions)
+
+
+def dump_outputs(out_dir: str, poses, frames) -> None:
+    """Writes frames (host 0x00RRGGBB arrays of one size) for output-for-output comparison of two builds:
+    frames.npy (len(frames), S) float32, which holds every 24-bit pixel exactly; pixel_index.npy (S,) their row-major
+    positions; poses.npy the drift-path pose of each frame.  S is every pixel when that fits DUMP_BYTES, else a fixed,
+    seeded sample of positions, the same in every frame."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = frames[0].size
+    s = min(n, DUMP_BYTES // (4 * len(frames) + 8))
+    idx = np.arange(n) if s == n else np.sort(np.random.default_rng(0).choice(n, s, replace=False))
+    np.save(os.path.join(out_dir, "frames.npy"), np.stack([f.reshape(-1)[idx] for f in frames]).astype(np.float32))
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "poses.npy"), np.asarray(poses, np.float64))
+
+
 def frame_digest(frame: np.ndarray) -> dict:
     a = np.ascontiguousarray(frame, np.uint32)
     return {"sum": int(a.sum(dtype=np.uint64)), "crc32": int(zlib.crc32(a.tobytes()))}
@@ -369,7 +386,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames of the last step that the output still holds (N = 1: the "
+                         "ring's, N > 1: the assembled last pose) to DIR as .npy, a seeded pixel sample where they exceed 48 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -563,7 +585,15 @@ def main():
 
     # ---- checks (untimed): the assembled frame equals the whole frame; digest of pose 0 for the cross-arm comparison
     whole_last = r.render(mats[POSES - 1], W, H)[0]
-    same = bool(np.array_equal(assembled[0](), whole_last))
+    last_frame = assembled[0]()
+    same = bool(np.array_equal(last_frame, whole_last))
+    if args.dump_outputs and rank == 0:
+        if world == 1:
+            held = min(args.ring, POSES)
+            dump_outputs(args.dump_outputs, range(POSES - held, POSES),
+                         [ring[(k[0] - held + j) % args.ring].cpu().numpy().view(np.uint32) for j in range(held)])
+        else:
+            dump_outputs(args.dump_outputs, [POSES - 1], [last_frame])
     banded_equals_whole = bool(max_over_ranks(0.0 if same else 1.0) == 0.0)
     frame0 = frame_digest(r.render(mats[0], W, H)[0])
     stats_last = r.stats(0)
@@ -701,7 +731,7 @@ def run_c2(args, r, rank, local_rank, world, dev, stream, barrier, max_over_rank
     import torch
     from swift3drenderer_b200 import assets, renderer as R, scene as S
     W, H, F, vpl = args.width, args.height, args.c2_frames, args.c2_views_per_launch
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     data_bin = assets.ensure_shipped_data_bin()
     sc = S.read_data_bin(data_bin)
     counts = sc.counts()

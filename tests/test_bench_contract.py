@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -56,3 +57,42 @@ def test_product_arm_needs_a_gpu():
     p = _run(["--steps", "1", "--warmup", "3", "--c3-solids", "100"])
     assert p.returncode != 0 and "no CUDA device" in (p.stderr + p.stdout)
     assert not [l for l in p.stdout.splitlines() if l.startswith("{")]   # no result line from a run that did not happen
+
+
+def test_dump_outputs_writes_exact_float32_frames_and_a_fixed_sample(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(5)
+    frames = [rng.integers(0, 1 << 24, (90, 160), dtype=np.uint32) for _ in range(3)]
+    bench.dump_outputs(str(tmp_path / "whole"), [5, 6, 7], frames)
+    got = np.load(tmp_path / "whole" / "frames.npy")
+    assert got.dtype == np.float32 and np.array_equal(got.astype(np.uint32), np.stack(frames).reshape(3, -1))
+    assert np.load(tmp_path / "whole" / "poses.npy").tolist() == [5, 6, 7]
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1000 * (4 * 3 + 8))   # room for 1 000 of the 14 400 pixels of each frame
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), [5, 6, 7], frames)
+    idx = np.load(tmp_path / "a" / "pixel_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 1000 and np.array_equal(idx, np.load(tmp_path / "b" / "pixel_index.npy"))
+    sample = np.load(tmp_path / "a" / "frames.npy")
+    assert np.array_equal(sample, np.load(tmp_path / "b" / "frames.npy"))
+    assert np.array_equal(sample.astype(np.uint32), np.stack(frames).reshape(3, -1)[:, idx.astype(np.int64)])
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_oracles_frames(tmp_path, oracle_port):
+    """--dump-outputs holds what the timed steps rendered: the frames of the last step still in the output ring."""
+    p = _run(["--steps", "2", "--warmup", "3", "--c3-solids", "2000", "--width", "640", "--height", "360",
+              "--no-cpu", "--no-e2e", "--no-secondary", "--dump-outputs", str(tmp_path)])
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 2
+    sys.path.insert(0, ROOT)
+    import bench
+    frames = np.load(tmp_path / "frames.npy")
+    idx = np.load(tmp_path / "pixel_index.npy").astype(np.int64)
+    poses = np.load(tmp_path / "poses.npy").astype(np.int64).tolist()
+    assert frames.dtype == np.float32 and poses == [4, 5, 6, 7] and len(idx) == 640 * 360
+    osc = oracle_port.OracleScene(path=bench.c3_data_bin(2000))
+    mats = oracle_port.camera_path(bench.drift_inputs(bench.POSES))
+    for got, pose in zip(frames, poses):
+        want = osc.render(mats[pose], 640, 360)["pixels"].reshape(-1)[idx]
+        assert np.array_equal(got, want.astype(np.float32)), f"pose {pose}"

@@ -2,6 +2,7 @@
 import os
 
 import numpy as np
+import pytest
 
 from swift3drenderer_b200 import scene as S
 
