@@ -161,6 +161,8 @@ S3R_API int s3r_set_option(S3RRenderer *r, const char *name, int64_t value);
  *          "pack24" (1 = 24-bit pixel transport over PCIe for host renders, default), "host_bands" (raster/
  *          copy pipeline depth of host renders, default 8), "copy_threads" (staging -> caller copy workers),
  *          "setup_capacity" (test hook: shrink the survivor buffers to exercise regrowth),
+ *          "rowtab_capacity" (test hook: cap the general path's row-start table at this many floats per view, 0 = empty —
+ *          tile-path triangles that do not fit keep their exact jumps; < 0 = the default size),
  *          "clusters" (general path front: 1 = over the load-time clusters — batch / cluster rejection, per-warp vertex stage and
  *          front tests with raster-space vertices in shared memory only, direct walk from a candidate queue; 0 = vertex_stage +
  *          triangle_classify over the raw stream; 2 (default) = clusters for partitioned submissions — bands, interleaved rows —

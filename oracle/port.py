@@ -73,7 +73,7 @@ def lib():
         _lib.oracle_render.argtypes = [
             ctypes.POINTER(CScene), ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p,
             ctypes.c_void_p, ctypes.POINTER(CStats), ctypes.c_void_p, ctypes.c_size_t,
-            ctypes.POINTER(ctypes.c_size_t)]
+            ctypes.POINTER(ctypes.c_size_t), ctypes.c_void_p]
         _lib.oracle_render.restype = ctypes.c_int
         _lib.oracle_vertex_stage.argtypes = [ctypes.POINTER(CScene), ctypes.c_void_p, ctypes.c_uint32,
                                              ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p]
@@ -127,10 +127,14 @@ class OracleScene:
             self.c.vertices, self.c.vertex_indices = v.ctypes.data, vi.ctypes.data
             self.c.attributes, self.c.attribute_indices, self.c.texels = at.ctypes.data, ai.ctypes.data, tx.ctypes.data
 
-    def render(self, matrix, width: int, height: int, want_depth=False, want_setups=False, setup_cap=None):
+    def render(self, matrix, width: int, height: int, want_depth=False, want_setups=False, setup_cap=None,
+               want_winner=False):
+        """want_winner: also return "winner", per pixel the order key of the triangle that wrote it last (its own index,
+        or T + parent for a triangle appended by the clipper), 0xFFFFFFFF on background."""
         m = np.ascontiguousarray(matrix, "<f4")
         px = np.empty((height, width), np.uint32)
         depth = np.empty((height, width), np.float32) if want_depth else None
+        winner = np.empty((height, width), np.uint32) if want_winner else None
         st = CStats()
         setups = None
         n = ctypes.c_size_t(0)
@@ -140,7 +144,7 @@ class OracleScene:
         lib().oracle_render(ctypes.byref(self.c), m.ctypes.data, width, height, px.ctypes.data,
                             depth.ctypes.data if want_depth else None, ctypes.byref(st),
                             setups.ctypes.data if want_setups else None, len(setups) if want_setups else 0,
-                            ctypes.byref(n))
+                            ctypes.byref(n), winner.ctypes.data if want_winner else None)
         stats = {k: int(getattr(st, k)) for k in STATS_FIELDS}
         stats["scratch_overflow"] = int(st.scratch_overflow)
         out = {"pixels": px, "stats": stats}
@@ -148,6 +152,8 @@ class OracleScene:
             out["depth"] = depth
         if want_setups:
             out["setups"] = setups[: min(n.value, len(setups))]
+        if want_winner:
+            out["winner"] = winner
         return out
 
     def vertex_stage(self, matrix, width: int, height: int):

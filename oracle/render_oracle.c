@@ -291,7 +291,8 @@ static uint32_t pack_rgb(v3 c) { /* RGB(), render.cpp:8: each channel through (u
 }
 
 int oracle_render(const OracleScene *s, const float *m, uint32_t width, uint32_t height, uint32_t *pixels,
-                  float *depth_out, OracleStats *stats, OracleSetup *setups, size_t setup_cap, size_t *setup_count) {
+                  float *depth_out, OracleStats *stats, OracleSetup *setups, size_t setup_cap, size_t *setup_count,
+                  uint32_t *winner) {
     OracleStats st;
     memset(&st, 0, sizeof(st));
     size_t n_setups = 0;
@@ -318,6 +319,7 @@ int oracle_render(const OracleScene *s, const float *m, uint32_t width, uint32_t
 
     /* clears, render.cpp:281-282 */
     for (size_t i = 0; i < npix; i++) { depth[i] = 0.f; pixels[i] = kBackground; }
+    if (winner) { for (size_t i = 0; i < npix; i++) { winner[i] = 0xFFFFFFFFu; } }
 
     /* vertex + normal loops, render.cpp:285-292 */
     for (uint64_t i = 0; i < V; i++) {
@@ -392,12 +394,13 @@ int oracle_render(const OracleScene *s, const float *m, uint32_t width, uint32_t
             tpp[0] = (pay[0].x * dx[0] + pay[1].x * dx[1]) + pay[2].x * dx[2]; /* :350-352 */
             tpp[1] = (pay[0].y * dy[0] + pay[1].y * dy[1]) + pay[2].y * dy[2];
         }
+        /* in place: own index; appended: T + parent index (appended triangles run in parent order) */
+        const uint32_t tri = index / 3, t_in = (uint32_t)(I / 3);
+        const uint32_t order = tri < t_in ? tri : t_in + sc.spawn_parent[tri - t_in];
         if (setups && n_setups < setup_cap) {
             OracleSetup *o = &setups[n_setups];
             memset(o, 0, sizeof(*o));
-            const uint32_t tri = index / 3, t_in = (uint32_t)(I / 3);
-            /* in place: own index; appended: T + parent index (appended triangles run in parent order) */
-            o->order = tri < t_in ? tri : t_in + sc.spawn_parent[tri - t_in];
+            o->order = order;
             o->xmin = xmin; o->xmax = xmax; o->ymin = ymin; o->ymax = ymax; o->area = area;
             for (int k = 0; k < 3; k++) {
                 o->wstart[k] = ws[k]; o->dx[k] = dx[k]; o->dy[k] = dy[k]; o->rvz[k] = rvz[k];
@@ -412,6 +415,7 @@ int oracle_render(const OracleScene *s, const float *m, uint32_t width, uint32_t
         float w[3] = {ws[0], ws[1], ws[2]}, wy[3] = {ws[0], ws[1], ws[2]};
         for (uint32_t y = ymin; y <= ymax; y++) {
             uint32_t *prow = pixels + (size_t)y * width;
+            uint32_t *wrow = winner ? winner + (size_t)y * width : NULL;
             float *drow = depth + (size_t)y * width;
             for (uint32_t x = xmin; x <= xmax; x++) {
                 st.bbox_pixels++;
@@ -421,6 +425,7 @@ int oracle_render(const OracleScene *s, const float *m, uint32_t width, uint32_t
                     if (ooz > drow[x]) {
                         st.shaded_pixels++;
                         drow[x] = ooz;
+                        if (wrow) { wrow[x] = order; }
                         const float b0 = w[0] / ooz, b1 = w[1] / ooz, b2 = w[2] / ooz;
                         v3 p = v3_add(v3_add(v3_scale(cvz[0], b0), v3_scale(cvz[1], b1)), v3_scale(cvz[2], b2));
                         v3 pu = v3_unit(p);

@@ -98,6 +98,7 @@ struct S3RRenderer {
     DevBuf<uint2> raster_items;        // ... and the tile kernel's work queue
     DevBuf<unsigned long long> pstate; // weights of the tile kernel's winners: 3 tagged words per pixel
     int opt_flat_max = 128;
+    int64_t rowtab_limit = -1;         // test hook "rowtab_capacity": floats of row-start table per view (< 0: no limit)
     uint32_t items_cap = 0;
     DevBuf<uint32_t> worklist;
     DevBuf<uint32_t> sticky;
@@ -745,7 +746,8 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     if (!f.direct_bin && r->opt_spans) {
         // general path: 8 M floats of row-start blocks per view; a triangle that does not fit keeps its exact jumps
         f.rowtab_cap = (uint32_t)std::min<size_t>(8u << 20, ((size_t)256 << 20) / std::max<size_t>(r->views_cap, 1));   // <= 1 GB in all
-        CUDA_TRY(r->rowtab.ensure((size_t)f.rowtab_cap * r->views_cap));
+        if (r->rowtab_limit >= 0) { f.rowtab_cap = (uint32_t)std::min<int64_t>(f.rowtab_cap, r->rowtab_limit); }
+        CUDA_TRY(r->rowtab.ensure(std::max<size_t>(1, (size_t)f.rowtab_cap * r->views_cap)));   // (an empty table still exists: its triangles jump)
         CUDA_TRY(r->rowbase.ensure((size_t)r->setup_cap * r->views_cap));
         f.rowtab = r->rowtab.p; f.rowbase = r->rowbase.p;
     }
@@ -852,7 +854,9 @@ static int finish_on(S3RRenderer *r, cudaStream_t s) {
     if (overflow & 2u) { r->tile_cap = std::max(r->tile_cap, need_entries + need_entries / 2 + 64); r->entries.release(); }
     if (overflow & 4u) { r->big_cap = std::max(r->big_cap, need_big + need_big / 2 + 64); r->big_list.release(); }
     if (overflow & 8u) {
-        r->walk_cap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(r->T, 1), (uint64_t)need_walk + need_walk / 4 + 1024);
+        // (not bounded by T: the front reserves the queue in per-warp chunks of 64 and pads them with holes, so a scene whose
+        // triangles nearly all take the direct walk needs more records than it has triangles)
+        r->walk_cap = (uint32_t)std::min<uint64_t>(0xFFFFFFFFull, (uint64_t)need_walk + need_walk / 4 + 1024);
         r->walk_q.release();
     }
     return 1;
@@ -1250,6 +1254,9 @@ extern "C" int s3r_set_option(S3RRenderer *r, const char *name, int64_t value) {
         r->setup_cap = (uint32_t)value; r->tile_cap = 4; r->big_cap = 4; r->walk_cap = 8; r->walk_q.release();
         r->vis.release(); r->shade.release(); r->head.release(); r->slot_of.release(); r->entries.release(); r->big_list.release(); r->rowbase.release();
         return S3R_OK;
+    }
+    if (!strcmp(name, "rowtab_capacity")) {   // test hook: row-start table size in floats per view (0: empty, < 0: default)
+        r->rowtab_limit = value; return S3R_OK;
     }
     return fail(S3R_E_ARG, std::string("unknown option ") + name);
 }
