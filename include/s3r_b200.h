@@ -153,13 +153,19 @@ S3R_API int s3r_set_option(S3RRenderer *r, const char *name, int64_t value);
 /* options: "tma_store" (1 = cp.async.bulk tile write-out, default; 0 = plain stores),
  *          "pin_host" (1 = cudaHostRegister the caller's frame buffers; default 0 — only for callers that
  *                      keep the buffer mapped while they pass it; drop-in: env S3R_PIN_HOST=1),
- *          "views_per_chunk" (views per kernel launch set, default 256), "timing" (per-stage and per-kernel events; n > 1: on every n-th submission only),
+ *          "views_per_chunk" (views per kernel launch set, default 256), "timing" (per-stage and per-kernel events, default 0
+ *          = off; n > 1: on every n-th submission only),
  *          "fused_small" (1 = one fused geometry CTA per view for scenes of at most 1920 triangles, default),
+ *          "direct_small" (general path: 1 = small unclipped survivors are walked by the classify kernel without a setup
+ *          record, default; 0 = every survivor is recorded),
+ *          "flat_max" (general path: recorded triangles whose box is under flat_max x flat_max pixels are walked flat, larger
+ *          ones by tiles; 16 .. 65536, default 128),
  *          "tensor_store" (1 = tile_raster writes each tile with one TMA tensor store instead of 32 bulk row copies, default),
  *          "spans" (1 = small scenes, whole-frame launches: the row walks of the largest survivors are done once per
  *          frame by span_walk instead of by exact jumps in every tile, default),
  *          "pack24" (1 = 24-bit pixel transport over PCIe for host renders, default), "host_bands" (raster/
- *          copy pipeline depth of host renders, default 8), "copy_threads" (staging -> caller copy workers),
+ *          copy pipeline depth of host renders, default 12), "copy_threads" (staging -> caller copy workers; default 0 =
+ *          min(14, hardware threads - 2)),
  *          "setup_capacity" (test hook: shrink the survivor buffers to exercise regrowth),
  *          "rowtab_capacity" (test hook: cap the general path's row-start table at this many floats per view, 0 = empty —
  *          tile-path triangles that do not fit keep their exact jumps; < 0 = the default size),

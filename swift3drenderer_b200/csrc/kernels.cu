@@ -2311,7 +2311,6 @@ static inline void mark(const LaunchMarks *m, const char *kernel) { if (m) { m->
 
 // Launch with programmatic stream serialization (see wait_for_predecessor): `after_kernel` = the previous operation in the
 // stream is one of this path's kernels.
-static int g_pdl = 1;
 template <typename... KArgs, typename... Args>
 static void launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool after_kernel, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -2321,10 +2320,9 @@ static void launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     // (not on the legacy / per-thread default streams: their implicit synchronisation and the programmatic edge do not mix)
     const bool real_stream = s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread;
-    cfg.attrs = attr; cfg.numAttrs = (g_pdl && after_kernel && real_stream) ? 1u : 0u;
+    cfg.attrs = attr; cfg.numAttrs = (after_kernel && real_stream) ? 1u : 0u;
     cudaLaunchKernelEx(&cfg, kernel, args...);
 }
-void set_dependent_launch(int on) { g_pdl = on; }
 
 int launch_geometry(const Frame &f, cudaStream_t s, const LaunchMarks *m) {
     int launches = 0;

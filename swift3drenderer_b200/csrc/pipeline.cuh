@@ -186,7 +186,6 @@ int launch_geometry(const Frame &f, cudaStream_t s, const LaunchMarks *marks = n
 int launch_raster(const Frame &f, cudaStream_t s, const LaunchMarks *marks = nullptr);     // per-tile visibility + shading + write-out
 int launch_geometry_small(const Frame &f, cudaStream_t s, const LaunchMarks *marks = nullptr);  // single-CTA-per-view fused geometry (+ span_walk when f.coltab is set)
 void launch_vertex_stage(const Frame &f, cudaStream_t s);   // vertex stage alone into f.rv (raster-vertex dumps)
-void set_dependent_launch(int on);   // programmatic dependent launch between the general path's kernels (default on)
 cudaError_t configure_kernels();
 void launch_exact_math(uint32_t mode, unsigned long long lo, unsigned long long count, uint32_t seed, unsigned long long *result,
                        cudaStream_t st);

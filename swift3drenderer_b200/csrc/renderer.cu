@@ -50,10 +50,15 @@ static int fail(int code, const std::string &msg) {
         }                                                                                                \
     } while (0)
 
+// A device allocation owned by its holder: grown by ensure(), freed with the holder (on the current device).
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
     size_t n = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept { *this = std::move(o); }
+    DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~DevBuf() { if (p) { cudaFree(p); } }
     cudaError_t ensure(size_t count) {
         if (count <= n) { return cudaSuccess; }
         if (p) { cudaFree(p); p = nullptr; n = 0; }
@@ -61,10 +66,68 @@ struct DevBuf {
         if (e == cudaSuccess) { n = count; }
         return e;
     }
-    void release() { if (p) { cudaFree(p); } p = nullptr; n = 0; }
 };
 
-struct HostPin { const void *ptr; size_t bytes; };
+// Registrations of caller frame buffers (cudaHostRegister with `flags`), so that their device->host copies run at full
+// PCIe rate.  A buffer seen before is looked up; a new one (or a resize, main.swift:156-165) first drops the registrations
+// it overlaps, and a ninth drops them all.  pin() returns false when the registration fails: copy through staging.
+struct HostPins {
+    struct Pin { const void *ptr; size_t bytes; };
+    unsigned flags;
+    std::vector<Pin> pins;
+    explicit HostPins(unsigned f) : flags(f) {}
+    bool pin(const void *ptr, size_t bytes) {
+        for (auto &p : pins) {
+            if (p.ptr == ptr && p.bytes >= bytes) { return true; }
+        }
+        for (size_t i = 0; i < pins.size();) {
+            const char *a = static_cast<const char *>(pins[i].ptr), *b = static_cast<const char *>(ptr);
+            if (a < b + bytes && b < a + pins[i].bytes) {
+                cudaHostUnregister(const_cast<void *>(pins[i].ptr));
+                pins.erase(pins.begin() + (long)i);
+            } else {
+                i++;
+            }
+        }
+        if (pins.size() >= 8) { clear(); }
+        if (cudaHostRegister(const_cast<void *>(ptr), bytes, flags) != cudaSuccess) {
+            cudaGetLastError();  // clear; fall back to a pageable copy
+            return false;
+        }
+        pins.push_back(Pin{ptr, bytes});
+        return true;
+    }
+    void clear() {
+        for (auto &p : pins) { cudaHostUnregister(const_cast<void *>(p.ptr)); }
+        pins.clear();
+    }
+};
+
+// Per-view scratch of the loaded scene's submissions: capacities and buffers, sized by ensure_scratch and dropped as a
+// whole when a scene is loaded.
+struct FrameScratch {
+    uint32_t views_cap = 0, tile_stride = 0;
+    uint32_t setup_cap = 0, tile_cap = 0, big_cap = 0, items_cap = 0;
+    uint32_t walk_cap = 0;
+    DevBuf<uint4> cluster_list;
+    DevBuf<uint8_t> walk_q;            // candidate queue of the direct walk: 40-byte records (front kernel -> walk kernel)
+    DevBuf<float4> rv;
+    DevBuf<SetupVis> vis;
+    DevBuf<SetupShade> shade;
+    DevBuf<uint4> head;
+    DevBuf<uint32_t> slot_of;
+    DevBuf<unsigned long long> keys;   // general path: per-pixel depth keys ...
+    DevBuf<uint2> raster_items;        // ... and the tile kernel's work queue
+    DevBuf<unsigned long long> pstate; // weights of the tile kernel's winners: 3 tagged words per pixel
+    DevBuf<uint32_t> worklist;
+    DevBuf<uint32_t> counters, big_list;   // counters: [views_cap][C_COUNT] followed by the tile histograms [views_cap][tile_stride]
+    DevBuf<uint32_t> entries;
+    DevBuf<float> cams;
+    DevBuf<float> coltab;     // small scenes: tile-column checkpoints of the largest survivors (span_walk)
+    DevBuf<uint32_t> span_slots;
+    DevBuf<float> rowtab;     // general path: row-start blocks of the tile-path triangles (post_setup)
+    DevBuf<uint32_t> rowbase;
+};
 
 struct S3RRenderer {
     int device = 0;
@@ -79,39 +142,17 @@ struct S3RRenderer {
     DevBuf<uint4> cl_hdr;
     DevBuf<float> cl_px, cl_py, cl_pz;
     DevBuf<uint32_t> cl_tri;
-    DevBuf<uint4> cluster_list;
-    DevBuf<uint8_t> walk_q;            // candidate queue of the direct walk: 40-byte records (front kernel -> walk kernel)
-    uint32_t walk_cap = 0;
     uint32_t n_clusters = 0;
     int opt_clusters = 2, opt_cluster_cull = 1;   // clusters: 0 off, 1 on, 2 on for partitioned submissions
     Frame last_frame;   // parameter block of the last submission (raster-vertex dumps on the cluster path)
-    // per-view scratch
-    uint32_t views_cap = 0, tile_stride = 0;
-    uint32_t setup_cap = 0, tile_cap = 0, big_cap = 0;
+    FrameScratch scratch;
     uint32_t views_per_chunk = 256;
-    DevBuf<float4> rv;
-    DevBuf<SetupVis> vis;
-    DevBuf<SetupShade> shade;
-    DevBuf<uint4> head;
-    DevBuf<uint32_t> slot_of;
-    DevBuf<unsigned long long> keys;   // general path: per-pixel depth keys ...
-    DevBuf<uint2> raster_items;        // ... and the tile kernel's work queue
-    DevBuf<unsigned long long> pstate; // weights of the tile kernel's winners: 3 tagged words per pixel
     int opt_flat_max = 128;
     int64_t rowtab_limit = -1;         // test hook "rowtab_capacity": floats of row-start table per view (< 0: no limit)
-    uint32_t items_cap = 0;
-    DevBuf<uint32_t> worklist;
     DevBuf<uint32_t> sticky;
     uint32_t *sticky_host = nullptr;   // pinned mirror of `sticky`
     float factor_override = 0.f;   // drop-in path: the reference's stale-factor rule (render.cpp:276-279)
-    DevBuf<uint32_t> counters, big_list;   // counters: [views_cap][C_COUNT] followed by the tile histograms [views_cap][tile_stride]
-    DevBuf<uint32_t> entries;
-    DevBuf<float> cams;
     DevBuf<uint32_t> frame;   // internal device framebuffer for host renders (u32 pixels, or 3 bytes/pixel when packed)
-    DevBuf<float> coltab;     // small scenes: tile-column checkpoints of the largest survivors (span_walk)
-    DevBuf<uint32_t> span_slots;
-    DevBuf<float> rowtab;     // general path: row-start blocks of the tile-path triangles (post_setup)
-    DevBuf<uint32_t> rowbase;
     // submission ring: pinned camera staging + events, so the host can run RING chunks ahead
     static constexpr int RING = 16;
     float *cams_pinned = nullptr;     // RING x views_cap x 12
@@ -134,7 +175,7 @@ struct S3RRenderer {
     uint32_t last_views = 0, last_W = 0, last_H = 0;
     cudaStream_t last_stream = nullptr;   // stream of the last s3r_render_device submission
     uint64_t launches = 0;
-    int opt_tma = 1, opt_pin_host = 0;   // pinning caller memory is opt-in: see pin_host()
+    int opt_tma = 1, opt_pin_host = 0;   // pinning caller memory is opt-in: see s3r_render_host
     // staged host output (default path of s3r_render_host)
     cudaStream_t copy_stream = nullptr, aux_stream = nullptr;
     cudaEvent_t ev_geometry = nullptr;
@@ -144,7 +185,7 @@ struct S3RRenderer {
     size_t staging_bytes = 0;
     HostCopier *copier = nullptr;
     int opt_copy_threads = 0, opt_host_bands = 12, opt_pack24 = 1, opt_fused_small = 1, opt_direct_small = 1, opt_spans = 1, opt_tmap = 1, opt_band_taper = 1;
-    std::vector<HostPin> pins;
+    HostPins pins{cudaHostRegisterDefault};
     // fused frame assembly
     std::vector<void *> own_frames, opened_frames;
     uint32_t *peer_out[MAX_PEERS] = {};
@@ -155,6 +196,24 @@ struct S3RRenderer {
 // lifetime
 // --------------------------------------------------------------------------------------------------
 extern "C" const char *s3r_last_error(void) { return g_error.c_str(); }
+
+static int create_device_objects(S3RRenderer *r) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking));
+    for (int i = 0; i < S3RRenderer::RING; i++) {
+        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_cams[i], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreate(&r->ev_t0[i])); CUDA_TRY(cudaEventCreate(&r->ev_t1[i])); CUDA_TRY(cudaEventCreate(&r->ev_t2[i]));
+        for (int k = 0; k < S3RRenderer::MAX_MARKS; k++) { CUDA_TRY(cudaEventCreate(&r->ev_mark[i][k])); }
+    }
+    CUDA_TRY(cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&r->aux_stream, cudaStreamNonBlocking));
+    CUDA_TRY(cudaEventCreateWithFlags(&r->ev_geometry, cudaEventDisableTiming));
+    for (int i = 0; i < S3RRenderer::MAX_SLICES; i++) {
+        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_raster[i], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_copy[i], cudaEventDisableTiming));
+    }
+    CUDA_TRY(configure_kernels());
+    return S3R_OK;
+}
 
 extern "C" int s3r_create(S3RRenderer **out, int device) {
     if (!out) { return fail(S3R_E_ARG, "out is null"); }
@@ -169,47 +228,24 @@ extern "C" int s3r_create(S3RRenderer **out, int device) {
     CUDA_TRY(cudaSetDevice(device));
     S3RRenderer *r = new S3RRenderer();
     r->device = device;
-    CUDA_TRY(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking));
-    for (int i = 0; i < S3RRenderer::RING; i++) {
-        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_cams[i], cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreate(&r->ev_t0[i])); CUDA_TRY(cudaEventCreate(&r->ev_t1[i])); CUDA_TRY(cudaEventCreate(&r->ev_t2[i]));
-        for (int k = 0; k < S3RRenderer::MAX_MARKS; k++) { CUDA_TRY(cudaEventCreate(&r->ev_mark[i][k])); }
-    }
-    CUDA_TRY(cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamCreateWithFlags(&r->aux_stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaEventCreateWithFlags(&r->ev_geometry, cudaEventDisableTiming));
-    for (int i = 0; i < S3RRenderer::MAX_SLICES; i++) {
-        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_raster[i], cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&r->ev_copy[i], cudaEventDisableTiming));
-    }
+    const int rc = create_device_objects(r);
+    if (rc) { s3r_destroy(r); return rc; }   // (s3r_destroy skips what was not created)
     if (const char *env = getenv("S3R_COPY_THREADS")) { r->opt_copy_threads = atoi(env); }
     if (const char *env = getenv("S3R_HOST_BANDS")) { r->opt_host_bands = std::max(1, atoi(env)); }
     if (const char *env = getenv("S3R_BAND_TAPER")) { r->opt_band_taper = atoi(env) != 0; }
     if (const char *env = getenv("S3R_PACK24")) { r->opt_pack24 = atoi(env) != 0; }
-    CUDA_TRY(configure_kernels());
     *out = r;
     return S3R_OK;
 }
 
-static void unpin_all(S3RRenderer *r) {
-    for (auto &p : r->pins) { cudaHostUnregister(const_cast<void *>(p.ptr)); }
-    r->pins.clear();
-}
-
+// The renderer's device buffers are freed by their destructors, on the device set here.
 extern "C" void s3r_destroy(S3RRenderer *r) {
     if (!r) { return; }
     cudaSetDevice(r->device);
     cudaStreamSynchronize(r->stream);
     for (void *p : r->opened_frames) { cudaIpcCloseMemHandle(p); }
     for (void *p : r->own_frames) { cudaFree(p); }
-    unpin_all(r);
-    r->pos_x.release(); r->pos_y.release(); r->pos_z.release();
-    for (int k = 0; k < 3; k++) { r->vi[k].release(); r->ai[k].release(); }
-    r->cl_hdr.release(); r->cl_px.release(); r->cl_py.release(); r->cl_pz.release(); r->cl_tri.release(); r->cluster_list.release(); r->walk_q.release();
-    r->attr.release(); r->texels.release(); r->rv.release(); r->vis.release(); r->shade.release(); r->head.release(); r->slot_of.release(); r->worklist.release(); r->keys.release(); r->raster_items.release(); r->pstate.release();
-    r->counters.release();
-    r->big_list.release(); r->entries.release(); r->cams.release(); r->frame.release(); r->sticky.release();
-    r->coltab.release(); r->span_slots.release(); r->rowtab.release(); r->rowbase.release();
+    r->pins.clear();
     if (r->cams_pinned) { cudaFreeHost(r->cams_pinned); }
     delete r->copier;
     if (r->sticky_host) { cudaFreeHost(r->sticky_host); }
@@ -299,9 +335,7 @@ extern "C" int s3r_load_scene_arrays(S3RRenderer *r, const float *vertices, uint
     if (n_texels) { CUDA_TRY(cudaMemcpy(r->texels.p, texels, n_texels * 4, cudaMemcpyHostToDevice)); }
     r->V = V; r->Vpad = px.size(); r->I = I; r->T = T; r->A = A; r->n_texels = n_texels;
     r->has_scene = true;
-    r->views_cap = 0;  // scratch is re-sized on the next render
-    r->walk_q.release(); r->walk_cap = 0;
-    r->worklist.release(); r->setup_cap = 0; r->tile_cap = 0; r->vis.release(); r->shade.release(); r->head.release(); r->slot_of.release(); r->entries.release(); r->big_list.release(); r->rowbase.release();
+    r->scratch = FrameScratch();   // sized for the new scene by the next render
     return S3R_OK;
 }
 
@@ -470,7 +504,7 @@ extern "C" float s3r_factor(uint32_t height) { return kNear * (float)height / (2
 // Small scenes (2T <= SORT_CAP survivors at most) skip the bin arrays: one fused geometry CTA per view and
 // in-kernel per-tile collection in the rasteriser.
 static bool uses_direct_bin(const S3RRenderer *r) {
-    return r->opt_fused_small && 2ull * r->T <= (uint64_t)SORT_CAP && r->setup_cap >= 2ull * r->T;
+    return r->opt_fused_small && 2ull * r->T <= (uint64_t)SORT_CAP && r->scratch.setup_cap >= 2ull * r->T;
 }
 
 // The cluster front (batch_cull, cluster_cull, cluster_front, direct_walk) pays for itself when much of the scene can be
@@ -481,55 +515,113 @@ static bool uses_clusters(const S3RRenderer *r, bool partitioned) {
     return r->n_clusters > 0 && (r->opt_clusters == 1 || (r->opt_clusters == 2 && partitioned));
 }
 
-static int ensure_scratch(S3RRenderer *r, uint32_t views, uint32_t n_tiles, bool partitioned) {
+// Sizes every per-view buffer a submission needs and points `f` at them.  `f` arrives with the submission's geometry
+// (views, frame size, tiles, output and key-plane strides).  Capacities only grow here; finish_on and the
+// "setup_capacity" hook change them, and a buffer whose size expression then grows is reallocated on the next call.
+// banded: the tile rows are rasterised in several launches (host renders).
+static int ensure_scratch(S3RRenderer *r, Frame &f, bool partitioned, bool banded, cudaStream_t s) {
+    FrameScratch &b = r->scratch;
     const uint32_t T = (uint32_t)r->T;
-    if (r->setup_cap == 0) {
+    if (b.setup_cap == 0) {
         // survivors are usually a small share of 2T; start at T/4 (min 4096) and regrow on demand
-        r->setup_cap = (uint32_t)std::min<uint64_t>(2ull * T + 16, std::max<uint64_t>(4096, T / 4));
-        r->big_cap = std::max<uint32_t>(1024, r->setup_cap / 16u);
-        r->tile_cap = 0;
+        b.setup_cap = (uint32_t)std::min<uint64_t>(2ull * T + 16, std::max<uint64_t>(4096, T / 4));
+        b.big_cap = std::max<uint32_t>(1024, b.setup_cap / 16u);
+        b.tile_cap = 0;
     }
-    if (r->tile_cap == 0) {
+    if (b.tile_cap == 0) {
         // per-tile list capacity: 4x the average load, a power of two in [256, setup_cap]; regrown on overflow
-        uint64_t want = 4ull * r->setup_cap / std::max<uint32_t>(n_tiles, 1u), cap = 256;
+        uint64_t want = 4ull * b.setup_cap / std::max<uint32_t>(f.n_tiles, 1u), cap = 256;
         while (cap < want) { cap <<= 1; }
-        r->tile_cap = (uint32_t)std::min<uint64_t>(cap, std::max<uint32_t>(r->setup_cap, 256u));
+        b.tile_cap = (uint32_t)std::min<uint64_t>(cap, std::max<uint32_t>(b.setup_cap, 256u));
     }
-    const uint32_t tile_stride = ((n_tiles + 1 + 63) / 64) * 64;
-    if (views > r->views_cap || tile_stride > r->tile_stride) {
-        r->views_cap = std::max(views, r->views_cap);
-        r->tile_stride = std::max(tile_stride, r->tile_stride);
+    b.views_cap = std::max(f.n_views, b.views_cap);
+    b.tile_stride = std::max(((f.n_tiles + 1 + 63) / 64) * 64, b.tile_stride);
+    const size_t vc = b.views_cap;
+    // small scenes are launch-latency bound: one fused CTA per view and no bin arrays instead of eight
+    // launches; 2T <= SORT_CAP guarantees every raster CTA can hold the whole survivor list
+    f.direct_bin = uses_direct_bin(r) ? 1 : 0;
+    const bool front = !f.direct_bin && uses_clusters(r, partitioned);
+    if (!front) { CUDA_TRY(b.rv.ensure(vc * r->Vpad)); }   // the cluster front keeps raster-space vertices on chip
+    f.rv = front ? nullptr : b.rv.p;
+    CUDA_TRY(b.vis.ensure(vc * b.setup_cap));
+    CUDA_TRY(b.shade.ensure(vc * b.setup_cap));
+    CUDA_TRY(b.head.ensure(vc * b.setup_cap));
+    if (!f.direct_bin) {
+        CUDA_TRY(b.slot_of.ensure(vc * 2ull * std::max<uint64_t>(r->T, 1)));
     }
-    const size_t vc = r->views_cap;
-    if (uses_direct_bin(r) || !uses_clusters(r, partitioned)) { CUDA_TRY(r->rv.ensure(vc * r->Vpad)); }   // the cluster front keeps raster-space vertices on chip
-    CUDA_TRY(r->vis.ensure(vc * r->setup_cap));
-    CUDA_TRY(r->shade.ensure(vc * r->setup_cap));
-    CUDA_TRY(r->head.ensure(vc * r->setup_cap));
-    if (!uses_direct_bin(r)) {
-        CUDA_TRY(r->slot_of.ensure(vc * 2ull * std::max<uint64_t>(r->T, 1)));
-    }
-    CUDA_TRY(r->worklist.ensure(vc * std::max<uint64_t>(r->T, 1)));
+    CUDA_TRY(b.worklist.ensure(vc * std::max<uint64_t>(r->T, 1)));
+    f.vis = b.vis.p; f.shade = b.shade.p; f.head = b.head.p; f.slot_of = b.slot_of.p; f.worklist = b.worklist.p; f.setup_cap = b.setup_cap;
     // per-view counters and, right behind them, the per-tile histograms: the cluster path clears both with one memset
-    if (vc * (C_COUNT + (size_t)r->tile_stride) > r->counters.n) { CUDA_TRY(cudaStreamSynchronize(r->stream)); }
-    CUDA_TRY(r->counters.ensure(vc * (C_COUNT + (size_t)r->tile_stride)));
+    if (vc * (C_COUNT + (size_t)b.tile_stride) > b.counters.n) { CUDA_TRY(cudaStreamSynchronize(r->stream)); }
+    CUDA_TRY(b.counters.ensure(vc * (C_COUNT + (size_t)b.tile_stride)));
+    f.counters = b.counters.p;
+    f.tile_count = b.counters.p + vc * C_COUNT;
+    f.tile_stride = b.tile_stride;
     if (!r->sticky.p) {
         CUDA_TRY(r->sticky.ensure(8)); CUDA_TRY(cudaMemset(r->sticky.p, 0, 32));
         CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&r->sticky_host), 32));
         memset(r->sticky_host, 0, 32);
     }
+    f.sticky = r->sticky.p;
     // bin lists exist only for scenes that do not take the in-kernel collection path
-    if (!uses_direct_bin(r)) {
-        CUDA_TRY(r->entries.ensure(vc * (size_t)r->tile_stride * r->tile_cap));
-        r->items_cap = r->tile_stride * (1u + r->tile_cap / RASTER_CHUNK);   // every non-empty tile + every full chunk
-        CUDA_TRY(r->raster_items.ensure(vc * (size_t)r->items_cap));
+    if (!f.direct_bin) {
+        CUDA_TRY(b.entries.ensure(vc * (size_t)b.tile_stride * b.tile_cap));
+        b.items_cap = b.tile_stride * (1u + b.tile_cap / RASTER_CHUNK);   // every non-empty tile + every full chunk
+        CUDA_TRY(b.raster_items.ensure(vc * (size_t)b.items_cap));
     }
-    CUDA_TRY(r->big_list.ensure(vc * r->big_cap));
-    CUDA_TRY(r->cams.ensure(vc * 12));
+    f.entries = b.entries.p; f.tile_cap = b.tile_cap;
+    f.raster_items = b.raster_items.p; f.items_cap = b.items_cap;
+    CUDA_TRY(b.big_list.ensure(vc * b.big_cap));
+    f.big_list = b.big_list.p; f.big_cap = b.big_cap;
+    CUDA_TRY(b.cams.ensure(vc * 12));
+    f.cams = b.cams.p;
     if (r->cams_pinned_views < vc) {
         CUDA_TRY(cudaStreamSynchronize(r->stream));
         if (r->cams_pinned) { cudaFreeHost(r->cams_pinned); }
         CUDA_TRY(cudaMallocHost(&r->cams_pinned, (size_t)S3RRenderer::RING * vc * 12 * sizeof(float)));
         r->cams_pinned_views = vc;
+    }
+    if (front) {
+        f.cl_hdr = r->cl_hdr.p; f.cl_px = r->cl_px.p; f.cl_py = r->cl_py.p; f.cl_pz = r->cl_pz.p; f.cl_tri = r->cl_tri.p;
+        f.n_clusters = r->n_clusters; f.cluster_cull = r->opt_cluster_cull;
+        f.list_cap = r->n_clusters;
+        CUDA_TRY(b.cluster_list.ensure(vc * f.list_cap));
+        f.cluster_list = b.cluster_list.p;
+        // candidates of the direct walk: a quarter of the triangles to begin with, regrown on overflow
+        if (b.walk_cap == 0) { b.walk_cap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(r->T, 1), std::max<uint64_t>(4096, r->T / 4)); }
+        CUDA_TRY(b.walk_q.ensure(vc * b.walk_cap * 40u));
+        f.walk_q = reinterpret_cast<WalkRecord *>(b.walk_q.p); f.walk_cap = b.walk_cap;
+    }
+    if (!f.direct_bin) {   // general path: per-pixel keys and winners for the flat passes
+        // keys are all zero between frames: allocation clears them, shade_tiles clears what a frame has set.  The old
+        // plane may still be read by the submission before: wait for it before it is freed.
+        if ((size_t)f.n_views * f.key_view_stride + 2 > b.keys.n) {
+            CUDA_TRY(cudaStreamSynchronize(s));
+            CUDA_TRY(b.keys.ensure((size_t)f.n_views * f.key_view_stride + 2));
+            CUDA_TRY(cudaMemsetAsync(b.keys.p, 0, b.keys.n * sizeof(unsigned long long), s));
+        }
+        CUDA_TRY(b.pstate.ensure(3u * ((size_t)f.n_views * f.out_view_stride + 2)));
+        f.pstate = b.pstate.p;
+    }
+    f.keys = b.keys.p;
+    if (f.direct_bin && r->opt_spans && !banded) {
+        // whole-frame launches of a small scene: the largest survivors' row walks are done once per frame (span_walk)
+        // instead of by exact jumps in every tile.  The banded host path keeps the jumps: its first band must not wait.
+        f.span_h = (f.H + 31u) & ~31u;
+        const size_t per_view = (size_t)SPAN_MAX * f.tiles_x * 3u * f.span_h;
+        if (per_view * vc * sizeof(float) <= (size_t)1 << 30) {
+            CUDA_TRY(b.coltab.ensure(per_view * vc));
+            CUDA_TRY(b.span_slots.ensure((size_t)SPAN_MAX * vc));
+            f.coltab = b.coltab.p; f.span_slots = b.span_slots.p;
+        }
+    }
+    if (!f.direct_bin && r->opt_spans) {
+        // general path: 8 M floats of row-start blocks per view; a triangle that does not fit keeps its exact jumps
+        f.rowtab_cap = (uint32_t)std::min<size_t>(8u << 20, ((size_t)256 << 20) / std::max<size_t>(vc, 1));   // <= 1 GB in all
+        if (r->rowtab_limit >= 0) { f.rowtab_cap = (uint32_t)std::min<int64_t>(f.rowtab_cap, r->rowtab_limit); }
+        CUDA_TRY(b.rowtab.ensure(std::max<size_t>(1, (size_t)f.rowtab_cap * vc)));   // (an empty table still exists: its triangles jump)
+        CUDA_TRY(b.rowbase.ensure((size_t)b.setup_cap * vc));
+        f.rowtab = b.rowtab.p; f.rowbase = b.rowbase.p;
     }
     return S3R_OK;
 }
@@ -619,13 +711,16 @@ static void mark_kernel(void *ctx, const char *kernel) {
     if (n < S3RRenderer::MAX_MARKS && cudaEventRecord(m->r->ev_mark[m->slot][n], m->s) == cudaSuccess) { m->r->mark_name[m->slot][n++] = kernel; }
 }
 
-// raster_bands > 1: the tile rows are rasterised in that many launches, with r->ev_raster[b] recorded
-// after band b (used by the staged host path to start the D2H of a band while the next one renders);
-// band_rows[b] receives the first pixel row (relative to y0) after band b.
-static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0,
-                        uint32_t y1, uint32_t *dev_out, cudaStream_t s, int raster_bands = 1,
-                        uint32_t *band_rows = nullptr, bool packed24 = false, uint32_t row_stride = 1,
-                        uint32_t row_phase = 0, const std::function<int(int)> *after_band = nullptr) {
+// Called by a host render after band b's raster launch and the record of r->ev_raster[b]; end_row is the first pixel
+// row (relative to y0) after band b.
+typedef std::function<int(int b, uint32_t end_row)> BandFn;
+
+// One submission of n_views views: pixel rows [y0, y1) of the W x H frame, or (row_stride > 1; y0 = 0, y1 = H) the tile
+// rows a with a % row_stride == row_phase, compacted.  The tile rows are rasterised in raster_bands launches; with
+// after_band (host renders), r->ev_raster[b] is recorded after band b and after_band runs.
+static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
+                        uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, cudaStream_t s, int raster_bands = 1,
+                        bool packed24 = false, const BandFn &after_band = nullptr) {
     Frame f;
     memset(&f, 0, sizeof(f));
     f.tiles_x = (W + TILE_W - 1) / TILE_W;
@@ -639,8 +734,12 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
         f.tiles_y = rows > row_phase ? (rows - row_phase + row_stride - 1) / row_stride : 0;
     }
     f.n_tiles = f.tiles_x * f.tiles_y;
+    f.n_views = n_views;
+    f.W = W; f.H = H; f.y0 = y0; f.y1 = y1;
+    f.out_view_stride = row_stride == 1 ? (unsigned long long)W * (y1 - y0) : (unsigned long long)W * f.tiles_y * TILE_H;
+    f.key_view_stride = (unsigned long long)W * (((f.out_view_stride / W) + 3u) & ~3ull);   // key plane: columns of 4 output rows
     const bool partitioned = row_stride > 1 || y0 > 0 || y1 < H;
-    int rc = ensure_scratch(r, n_views, f.n_tiles, partitioned);
+    int rc = ensure_scratch(r, f, partitioned, raster_bands > 1, s);
     if (rc) { return rc; }
     const int slot = (int)(r->chunk_counter++ % S3RRenderer::RING);
     if (r->slot_used[slot]) {  // the chunk that used this slot RING submissions ago
@@ -658,7 +757,7 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     } else {
         float *staging = r->cams_pinned + (size_t)slot * r->cams_pinned_views * 12;
         memcpy(staging, cams, (size_t)n_views * 12 * sizeof(float));
-        CUDA_TRY(cudaMemcpyAsync(r->cams.p, staging, (size_t)n_views * 12 * sizeof(float), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(r->scratch.cams.p, staging, (size_t)n_views * 12 * sizeof(float), cudaMemcpyHostToDevice, s));
         CUDA_TRY(cudaEventRecord(r->ev_cams[slot], s));
         r->slot_used[slot] = true;
     }
@@ -674,83 +773,24 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     f.attr = r->attr.p; f.texels = r->texels.p;
     f.V = (uint32_t)r->V; f.Vpad = (uint32_t)r->Vpad; f.T = (uint32_t)r->T; f.A = (uint32_t)r->A;
     f.n_tex = std::max<uint32_t>(1, (uint32_t)(r->n_texels >> 18));
-    f.cams = r->cams.p; f.n_views = n_views;
-    f.W = W; f.H = H; f.y0 = y0; f.y1 = y1;
     f.fw = (float)W; f.fh = (float)H; f.half_w = f.fw / 2; f.half_h = f.fh / 2;  // screen_size / 2, render.cpp:284,288
     f.factor = r->factor_override != 0.f ? r->factor_override : s3r_factor(H);
-    f.rv = r->rv.p;
-    if (!uses_direct_bin(r) && uses_clusters(r, partitioned)) {
-        f.cl_hdr = r->cl_hdr.p; f.cl_px = r->cl_px.p; f.cl_py = r->cl_py.p; f.cl_pz = r->cl_pz.p; f.cl_tri = r->cl_tri.p;
-        f.n_clusters = r->n_clusters; f.cluster_cull = r->opt_cluster_cull;
-        f.list_cap = r->n_clusters;
-        CUDA_TRY(r->cluster_list.ensure((size_t)r->views_cap * f.list_cap));
-        f.cluster_list = r->cluster_list.p;
-        // candidates of the direct walk: a quarter of the triangles to begin with, regrown on overflow
-        if (r->walk_cap == 0) { r->walk_cap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(r->T, 1), std::max<uint64_t>(4096, r->T / 4)); }
-        CUDA_TRY(r->walk_q.ensure((size_t)r->views_cap * r->walk_cap * 40u));
-        f.walk_q = reinterpret_cast<WalkRecord *>(r->walk_q.p); f.walk_cap = r->walk_cap;
-        f.rv = nullptr;
-    }
-    f.vis = r->vis.p; f.shade = r->shade.p; f.head = r->head.p; f.slot_of = r->slot_of.p; f.worklist = r->worklist.p; f.setup_cap = r->setup_cap;
     f.band_lo = (float)y0; f.band_hi = (float)y1;
-    f.counters = r->counters.p;
-    f.sticky = r->sticky.p;
-    f.tile_count = r->counters.p + (size_t)r->views_cap * C_COUNT;
-    f.tile_stride = r->tile_stride;
-    f.entries = r->entries.p; f.tile_cap = r->tile_cap;
-    f.raster_items = r->raster_items.p; f.items_cap = r->items_cap;
-    f.big_list = r->big_list.p; f.big_cap = r->big_cap;
     f.out = dev_out;
     f.n_peers = r->n_peers;
     for (uint32_t k = 0; k < r->n_peers; k++) { f.peer_out[k] = r->peer_out[k]; }
-    f.keys = r->keys.p;
-    f.out_view_stride = row_stride == 1 ? (unsigned long long)W * (y1 - y0) : (unsigned long long)W * f.tiles_y * TILE_H;
-    f.key_view_stride = (unsigned long long)W * (((f.out_view_stride / W) + 3u) & ~3ull);   // key plane: columns of 4 output rows
-    if (!uses_direct_bin(r)) {   // general path: per-pixel keys and winners for the flat passes
-        // keys are all zero between frames: allocation clears them, shade_tiles clears what a frame has set
-        if ((size_t)n_views * f.key_view_stride + 2 > r->keys.n) {
-            CUDA_TRY(cudaStreamSynchronize(s));
-            CUDA_TRY(r->keys.ensure((size_t)n_views * f.key_view_stride + 2));
-            CUDA_TRY(cudaMemsetAsync(r->keys.p, 0, r->keys.n * sizeof(unsigned long long), s));
-        }
-        f.keys = r->keys.p;
-        CUDA_TRY(r->pstate.ensure(3u * ((size_t)n_views * f.out_view_stride + 2)));
-        f.pstate = r->pstate.p;
-    }
     f.out_packed24 = packed24 ? 1 : 0;
     f.use_tma = r->opt_tma && (W % (packed24 ? 16 : 4) == 0) && ((reinterpret_cast<uintptr_t>(dev_out) & 15u) == 0);
     // (interleaved tile rows keep the row copies: rows past H stay unwritten; so do bands that start inside a tile row —
     // the store's start coordinate must not be negative)
-    if (f.use_tma && r->opt_tmap && uses_direct_bin(r) && dev_out && row_stride == 1 && y0 % TILE_H == 0) {
+    if (f.use_tma && r->opt_tmap && f.direct_bin && dev_out && row_stride == 1 && y0 % TILE_H == 0) {
         f.use_tmap = encode_out_map(&f.out_map, dev_out, W, (uint64_t)(f.out_view_stride / W), n_views, f.out_view_stride, packed24) ? 1 : 0;
     }
     if (timed) { CUDA_TRY(cudaEventRecord(r->ev_t0[slot], s)); }
-    // small scenes are launch-latency bound: one fused CTA per view and no bin arrays instead of eight
-    // launches; 2T <= SORT_CAP guarantees every raster CTA can hold the whole survivor list
-    f.direct_bin = uses_direct_bin(r) ? 1 : 0;
     if (f.n_peers && (f.direct_bin || packed24)) { return fail(S3R_E_ARG, "peer frames need the general path (scene over 1920 triangles) and device output"); }
     f.direct_small = !f.direct_bin && r->opt_direct_small ? 1 : 0;
     f.flat_max = (uint32_t)r->opt_flat_max;
     f.rs_magic = row_stride > 1 ? (uint32_t)((1ull << 32) / row_stride) + 1u : 0u;
-    if (f.direct_bin && r->opt_spans && raster_bands <= 1) {
-        // whole-frame launches of a small scene: the largest survivors' row walks are done once per frame (span_walk)
-        // instead of by exact jumps in every tile.  The banded host path keeps the jumps: its first band must not wait.
-        f.span_h = (H + 31u) & ~31u;
-        const size_t per_view = (size_t)SPAN_MAX * f.tiles_x * 3u * f.span_h;
-        if (per_view * r->views_cap * sizeof(float) <= (size_t)1 << 30) {
-            CUDA_TRY(r->coltab.ensure(per_view * r->views_cap));
-            CUDA_TRY(r->span_slots.ensure((size_t)SPAN_MAX * r->views_cap));
-            f.coltab = r->coltab.p; f.span_slots = r->span_slots.p;
-        }
-    }
-    if (!f.direct_bin && r->opt_spans) {
-        // general path: 8 M floats of row-start blocks per view; a triangle that does not fit keeps its exact jumps
-        f.rowtab_cap = (uint32_t)std::min<size_t>(8u << 20, ((size_t)256 << 20) / std::max<size_t>(r->views_cap, 1));   // <= 1 GB in all
-        if (r->rowtab_limit >= 0) { f.rowtab_cap = (uint32_t)std::min<int64_t>(f.rowtab_cap, r->rowtab_limit); }
-        CUDA_TRY(r->rowtab.ensure(std::max<size_t>(1, (size_t)f.rowtab_cap * r->views_cap)));   // (an empty table still exists: its triangles jump)
-        CUDA_TRY(r->rowbase.ensure((size_t)r->setup_cap * r->views_cap));
-        f.rowtab = r->rowtab.p; f.rowbase = r->rowbase.p;
-    }
     r->launches += (uint64_t)(f.direct_bin ? launch_geometry_small(f, s, mk) : launch_geometry(f, s, mk));
     if (r->sticky_host) {
         // overflow record of this submission, read back on a side stream behind the geometry kernels: a 16-byte copy IN the
@@ -763,20 +803,18 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     // (general path: the tile kernel runs with the first band over the whole frame, the bands cut the shading pass)
     const int nb = std::max(1, std::min<int>(raster_bands, (int)f.tiles_y));
     uint32_t edge[S3RRenderer::MAX_SLICES + 1];
-    const int n_edges = band_edges(f.tiles_y, nb, r->opt_band_taper && after_band, edge);
+    const int n_edges = band_edges(f.tiles_y, nb, r->opt_band_taper && after_band != nullptr, edge);
     for (int b = 0; b + 1 < n_edges; b++) {
         f.raster_row0 = edge[b];
         f.raster_rows = edge[b + 1] - edge[b];
         r->launches += (uint64_t)launch_raster(f, s, mk);
-        if (raster_bands > 1 || band_rows) {
-            CUDA_TRY(cudaEventRecord(r->ev_raster[b], s));
-            if (band_rows) {
-                const uint32_t end_row = (f.tile_row0 + f.raster_row0 + f.raster_rows) * TILE_H;
-                band_rows[b] = std::min(y1, std::max(y0, end_row)) - y0;
-            }
+        if (after_band) {
             // the host path enqueues band b's device->host copy right here, before the next band's launch call,
             // so that the link starts as early as the GPU allows
-            if (after_band) { int rc2 = (*after_band)(b); if (rc2) { return rc2; } }
+            CUDA_TRY(cudaEventRecord(r->ev_raster[b], s));
+            const uint32_t end_row = (f.tile_row0 + f.raster_row0 + f.raster_rows) * TILE_H;
+            int rc2 = after_band(b, std::min(y1, std::max(y0, end_row)) - y0);
+            if (rc2) { return rc2; }
         }
     }
     if (timed) { CUDA_TRY(cudaEventRecord(r->ev_t2[slot], s)); r->slot_timed[slot] = true; }
@@ -785,20 +823,24 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     return S3R_OK;
 }
 
-extern "C" int s3r_render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
-                                 uint32_t y0, uint32_t y1, uint32_t *dev_out, void *stream) {
+// The device entry points: validation, stream choice and the view-chunk loop.  row_stride == 1: pixel rows [y0, y1);
+// otherwise y0 = 0, y1 = H and the tile rows a with a % row_stride == row_phase.
+static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
+                         uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, void *stream) {
     if (!r || !cams || (!dev_out && r->n_peers == 0)) { return fail(S3R_E_ARG, "null argument"); }
     if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
-    if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0) {
+    if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0 || row_stride == 0 || row_phase >= row_stride) {
         return fail(S3R_E_ARG, "bad frame geometry");
     }
+    const uint32_t tile_rows = (H + TILE_H - 1) / TILE_H;
+    if (tile_rows <= row_phase) { return S3R_OK; }   // this phase owns no tile row
     CUDA_TRY(cudaSetDevice(r->device));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
     r->last_stream = s;
-    const size_t view_px = (size_t)W * (y1 - y0);
+    const size_t view_px = (size_t)W * (row_stride == 1 ? y1 - y0 : (tile_rows - row_phase + row_stride - 1) / row_stride * TILE_H);
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
-        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, dev_out + view_px * v0, s);
+        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, dev_out + view_px * v0, s);
         if (rc) { return rc; }
         r->last_views = nv;
     }
@@ -806,31 +848,17 @@ extern "C" int s3r_render_device(S3RRenderer *r, const float *cams, uint32_t n_v
     return S3R_OK;
 }
 
-extern "C" uint32_t s3r_tile_height(void) { return (uint32_t)TILE_H; }
+extern "C" int s3r_render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
+                                 uint32_t y0, uint32_t y1, uint32_t *dev_out, void *stream) {
+    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, dev_out, stream);
+}
 
 extern "C" int s3r_render_device_rows(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
                                       uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, void *stream) {
-    if (!r || !cams || (!dev_out && r->n_peers == 0)) { return fail(S3R_E_ARG, "null argument"); }
-    if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
-    if (W == 0 || H == 0 || W > 65535 || H > 65535 || n_views == 0 || row_stride == 0 || row_phase >= row_stride) {
-        return fail(S3R_E_ARG, "bad frame geometry");
-    }
-    if ((H + TILE_H - 1) / TILE_H <= row_phase) { return S3R_OK; }   // this phase owns no tile row
-    CUDA_TRY(cudaSetDevice(r->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
-    r->last_stream = s;
-    const uint32_t rows = (H + TILE_H - 1) / TILE_H, owned = (rows - row_phase + row_stride - 1) / row_stride;
-    const size_t view_px = (size_t)W * owned * TILE_H;
-    for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
-        const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
-        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, 0, H, dev_out + view_px * v0, s, 1, nullptr, false,
-                              row_stride, row_phase);
-        if (rc) { return rc; }
-        r->last_views = nv;
-    }
-    r->last_W = W; r->last_H = H;
-    return S3R_OK;
+    return render_device(r, cams, n_views, W, H, 0, H, row_stride, row_phase, dev_out, stream);
 }
+
+extern "C" uint32_t s3r_tile_height(void) { return (uint32_t)TILE_H; }
 
 // Waits for the renderer's work, reads the per-view counters back and regrows capacities.
 // Returns 1 if something overflowed (the frame(s) of the last chunk must be rendered again).
@@ -845,19 +873,17 @@ static int finish_on(S3RRenderer *r, cudaStream_t s) {
     if (!overflow) { return S3R_OK; }
     CUDA_TRY(cudaMemset(r->sticky.p, 0, sizeof(sticky)));
     memset(r->sticky_host, 0, sizeof(sticky));
+    FrameScratch &b = r->scratch;   // (ensure_scratch regrows the buffers whose size these capacities set)
     if (overflow & 1u) {
-        r->setup_cap = (uint32_t)std::min<uint64_t>(2ull * r->T + 16, (uint64_t)need_setups + need_setups / 2 + 1024);
-        r->big_cap = std::max(r->big_cap, r->setup_cap / 16u);
-        // vis/shade are view-strided by setup_cap: force reallocation
-        r->vis.release(); r->shade.release(); r->head.release(); r->slot_of.release(); r->entries.release(); r->big_list.release(); r->rowbase.release();
+        b.setup_cap = (uint32_t)std::min<uint64_t>(2ull * r->T + 16, (uint64_t)need_setups + need_setups / 2 + 1024);
+        b.big_cap = std::max(b.big_cap, b.setup_cap / 16u);
     }
-    if (overflow & 2u) { r->tile_cap = std::max(r->tile_cap, need_entries + need_entries / 2 + 64); r->entries.release(); }
-    if (overflow & 4u) { r->big_cap = std::max(r->big_cap, need_big + need_big / 2 + 64); r->big_list.release(); }
+    if (overflow & 2u) { b.tile_cap = std::max(b.tile_cap, need_entries + need_entries / 2 + 64); }
+    if (overflow & 4u) { b.big_cap = std::max(b.big_cap, need_big + need_big / 2 + 64); }
     if (overflow & 8u) {
         // (not bounded by T: the front reserves the queue in per-warp chunks of 64 and pads them with holes, so a scene whose
         // triangles nearly all take the direct walk needs more records than it has triangles)
-        r->walk_cap = (uint32_t)std::min<uint64_t>(0xFFFFFFFFull, (uint64_t)need_walk + need_walk / 4 + 1024);
-        r->walk_q.release();
+        b.walk_cap = (uint32_t)std::min<uint64_t>(0xFFFFFFFFull, (uint64_t)need_walk + need_walk / 4 + 1024);
     }
     return 1;
 }
@@ -865,35 +891,6 @@ static int finish_on(S3RRenderer *r, cudaStream_t s) {
 extern "C" int s3r_finish(S3RRenderer *r) {
     if (!r) { return fail(S3R_E_ARG, "renderer is null"); }
     return finish_on(r, r->last_stream ? r->last_stream : r->stream);
-}
-
-// OPT-IN ("pin_host" option / S3R_PIN_HOST=1): cudaHostRegister the caller's frame buffer so the D2H
-// copy runs at full PCIe rate.  Only safe when the caller keeps that allocation mapped for as long
-// as it passes it (the reference's main loop does: one double buffer, re-allocated on resize only,
-// main.swift:156-165).  A registration that outlives its memory poisons every later CUDA call that
-// touches a host pointer in the recycled range, so it is never done behind the caller's back.
-static bool pin_host(S3RRenderer *r, const void *ptr, size_t bytes) {
-    if (!r->opt_pin_host) { return false; }
-    for (auto &p : r->pins) {
-        if (p.ptr == ptr && p.bytes >= bytes) { return true; }
-    }
-    // a new buffer (or a resize, main.swift:156-165): drop stale registrations that overlap it
-    for (size_t i = 0; i < r->pins.size();) {
-        const char *a = static_cast<const char *>(r->pins[i].ptr), *b = static_cast<const char *>(ptr);
-        if (a < b + bytes && b < a + r->pins[i].bytes) {
-            cudaHostUnregister(const_cast<void *>(r->pins[i].ptr));
-            r->pins.erase(r->pins.begin() + (long)i);
-        } else {
-            i++;
-        }
-    }
-    if (r->pins.size() >= 8) { unpin_all(r); }
-    if (cudaHostRegister(const_cast<void *>(ptr), bytes, cudaHostRegisterDefault) != cudaSuccess) {
-        cudaGetLastError();  // clear; fall back to a pageable copy
-        return false;
-    }
-    r->pins.push_back(HostPin{ptr, bytes});
-    return true;
 }
 
 // A registration made for a caller's buffer goes stale if the caller unmaps that memory and later
@@ -935,7 +932,12 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
     if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0) { return fail(S3R_E_ARG, "bad frame geometry"); }
     CUDA_TRY(cudaSetDevice(r->device));
     const size_t view_px = (size_t)W * (y1 - y0);
-    const bool pinned = pin_host(r, host_out, view_px * n_views * 4);
+    // OPT-IN ("pin_host" option / S3R_PIN_HOST=1): cudaHostRegister the caller's frame buffer so the D2H
+    // copy runs at full PCIe rate.  Only safe when the caller keeps that allocation mapped for as long
+    // as it passes it (the reference's main loop does: one double buffer, re-allocated on resize only,
+    // main.swift:156-165).  A registration that outlives its memory poisons every later CUDA call that
+    // touches a host pointer in the recycled range, so it is never done behind the caller's back.
+    const bool pinned = r->opt_pin_host && r->pins.pin(host_out, view_px * n_views * 4);
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
         uint32_t *dst = host_out + view_px * v0;
@@ -949,7 +951,6 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
         bool rendered = false;
         for (int attempt = 0; attempt < 8 && !rendered; attempt++) {
             // ---- enqueue: geometry, banded raster, one D2H per band/slice on the copy stream -----
-            uint32_t band_rows[S3RRenderer::MAX_SLICES] = {};
             // band-pipelined raster (small scenes) or shading (general path) and copy: band k crosses PCIe while band k + 1 renders
             const int bands = nv == 1 ? std::max(1, std::min(r->opt_host_bands, S3RRenderer::MAX_SLICES)) : 1;
             std::vector<CopySlice> slices;
@@ -957,41 +958,27 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
             if (pinned) { plant_sentinels(dst, view_px * nv); }
             int n_ev = 0;
             uint32_t row = 0;
-            const std::function<int(int)> copy_band = [&](int b) -> int {   // one view: band b's copy follows its raster launch
-                const size_t pa = (size_t)row * W, pe = (size_t)band_rows[b] * W;
-                const size_t a = pa * bpp, e = pe * bpp;
-                row = band_rows[b];
+            // band b's pixels of all nv views; several views have one band, copied in slices of about 4 MB
+            const BandFn copy_band = [&](int b, uint32_t end_row) -> int {
+                const size_t pa = (size_t)row * W * nv, pe = (size_t)end_row * W * nv;
+                row = end_row;
                 CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, r->ev_raster[b], 0));
-                if (e > a) {
-                    CUDA_TRY(cudaMemcpyAsync(target + a, reinterpret_cast<uint8_t *>(r->frame.p) + a, e - a,
+                const size_t n_sl = nv == 1 ? 1 : std::min<size_t>(S3RRenderer::MAX_SLICES, std::max<size_t>(1, chunk_bytes >> 22));
+                for (size_t i = 0; i < n_sl; i++) {
+                    const size_t a = pa + (((pe - pa) * i / n_sl) & ~(size_t)63);
+                    const size_t e = i + 1 == n_sl ? pe : pa + (((pe - pa) * (i + 1) / n_sl) & ~(size_t)63);
+                    if (e <= a) { continue; }
+                    CUDA_TRY(cudaMemcpyAsync(target + a * bpp, reinterpret_cast<uint8_t *>(r->frame.p) + a * bpp, (e - a) * bpp,
                                              cudaMemcpyDeviceToHost, r->copy_stream));
                     CUDA_TRY(cudaEventRecord(r->ev_copy[n_ev], r->copy_stream));
-                    slices.push_back(CopySlice{r->staging + a, reinterpret_cast<uint8_t *>(dst) + pa * 4, pe - pa});
+                    slices.push_back(CopySlice{r->staging + a * bpp, reinterpret_cast<uint8_t *>(dst) + a * 4, e - a});
                     n_ev++;
                 }
                 return S3R_OK;
             };
-            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, r->frame.p, r->stream, bands, band_rows, packed, 1, 0,
-                                  nv == 1 ? &copy_band : nullptr);
+            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, r->frame.p, r->stream, bands, packed, copy_band);
             if (rc) { return rc; }
             r->last_views = nv; r->last_W = W; r->last_H = H;
-            if (nv == 1) {
-                // (copies already enqueued band by band)
-            } else {
-                CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, r->ev_raster[0], 0));
-                const size_t total_px = view_px * nv;
-                const size_t n_sl = std::min<size_t>(S3RRenderer::MAX_SLICES, std::max<size_t>(1, chunk_bytes >> 22));
-                for (size_t i = 0; i < n_sl; i++) {
-                    const size_t pa = (total_px * i / n_sl) & ~(size_t)63;
-                    const size_t pe = i + 1 == n_sl ? total_px : (total_px * (i + 1) / n_sl) & ~(size_t)63;
-                    if (pe <= pa) { continue; }
-                    CUDA_TRY(cudaMemcpyAsync(target + pa * bpp, reinterpret_cast<uint8_t *>(r->frame.p) + pa * bpp, (pe - pa) * bpp,
-                                             cudaMemcpyDeviceToHost, r->copy_stream));
-                    CUDA_TRY(cudaEventRecord(r->ev_copy[n_ev], r->copy_stream));
-                    slices.push_back(CopySlice{r->staging + pa * bpp, reinterpret_cast<uint8_t *>(dst) + pa * 4, pe - pa});
-                    n_ev++;
-                }
-            }
             // ---- drain: as each slice lands in staging the worker threads move it to the caller ----
             if (!pinned) { r->copier->begin(&slices, packed); }
             cudaError_t ce = cudaSuccess;
@@ -1007,7 +994,7 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
             if (rc == 0) {
                 if (pinned && !sentinels_gone(dst, view_px * nv)) {
                     // stale registration: drop every pin and copy again through the pageable path
-                    unpin_all(r);
+                    r->pins.clear();
                     CUDA_TRY(cudaMemcpy(dst, r->frame.p, view_px * nv * 4, cudaMemcpyDeviceToHost));
                 }
                 rendered = true;
@@ -1090,7 +1077,7 @@ extern "C" int s3r_get_stats(S3RRenderer *r, uint32_t view, S3RStats *out) {
     if (view >= r->last_views) { return fail(S3R_E_ARG, "view out of range"); }
     CUDA_TRY(cudaSetDevice(r->device));
     uint32_t c[C_COUNT];
-    CUDA_TRY(cudaMemcpy(c, r->counters.p + (size_t)view * C_COUNT, sizeof(c), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(c, r->scratch.counters.p + (size_t)view * C_COUNT, sizeof(c), cudaMemcpyDeviceToHost));
     memset(out, 0, sizeof(*out));
     out->triangles_in = (uint32_t)r->T;
     out->near_rejected = c[C_NEAR]; out->clipped = c[C_CLIPPED]; out->spawned = c[C_SPAWNED]; out->culled = c[C_CULLED];
@@ -1106,14 +1093,14 @@ extern "C" int s3r_dump_raster_vertices(S3RRenderer *r, uint32_t view, float *ou
         // the frame went through the cluster front, which keeps raster-space vertices in shared memory: run the vertex
         // stage alone over the original vertex stream with the same camera, factor and frame size
         CUDA_TRY(cudaStreamSynchronize(r->last_stream ? r->last_stream : r->stream));
-        CUDA_TRY(r->rv.ensure((size_t)r->views_cap * r->Vpad));
+        CUDA_TRY(r->scratch.rv.ensure((size_t)r->scratch.views_cap * r->Vpad));
         Frame f = r->last_frame;
-        f.rv = r->rv.p; f.counters = nullptr; f.n_tiles = 0;
+        f.rv = r->scratch.rv.p; f.counters = nullptr; f.n_tiles = 0;
         launch_vertex_stage(f, r->stream);
         r->launches++;
         CUDA_TRY(cudaStreamSynchronize(r->stream));
     }
-    CUDA_TRY(cudaMemcpy(out, r->rv.p + (size_t)view * r->Vpad, r->V * sizeof(float4), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(out, r->scratch.rv.p + (size_t)view * r->Vpad, r->V * sizeof(float4), cudaMemcpyDeviceToHost));
     return S3R_OK;
 }
 
@@ -1122,14 +1109,14 @@ extern "C" int s3r_dump_setups(S3RRenderer *r, uint32_t view, S3RSetupDump *out,
     if (view >= r->last_views) { return fail(S3R_E_ARG, "view out of range"); }
     CUDA_TRY(cudaSetDevice(r->device));
     uint32_t n = 0;
-    CUDA_TRY(cudaMemcpy(&n, r->counters.p + (size_t)view * C_COUNT + C_SETUPS, 4, cudaMemcpyDeviceToHost));
-    n = std::min(n, r->setup_cap);
+    CUDA_TRY(cudaMemcpy(&n, r->scratch.counters.p + (size_t)view * C_COUNT + C_SETUPS, 4, cudaMemcpyDeviceToHost));
+    n = std::min(n, r->scratch.setup_cap);
     *count = n;
     if (!out || n == 0) { return S3R_OK; }
     std::vector<SetupVis> v(n);
     std::vector<SetupShade> s(n);
-    CUDA_TRY(cudaMemcpy(v.data(), r->vis.p + (size_t)view * r->setup_cap, n * sizeof(SetupVis), cudaMemcpyDeviceToHost));
-    CUDA_TRY(cudaMemcpy(s.data(), r->shade.p + (size_t)view * r->setup_cap, n * sizeof(SetupShade), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(v.data(), r->scratch.vis.p + (size_t)view * r->scratch.setup_cap, n * sizeof(SetupVis), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(s.data(), r->scratch.shade.p + (size_t)view * r->scratch.setup_cap, n * sizeof(SetupShade), cudaMemcpyDeviceToHost));
     std::vector<uint32_t> idx(n);
     for (uint32_t i = 0; i < n; i++) { idx[i] = i; }
     std::sort(idx.begin(), idx.end(), [&](uint32_t a, uint32_t b) { return v[a].order < v[b].order; });
@@ -1168,7 +1155,6 @@ extern "C" int s3r_debug_walk(S3RRenderer *r, const float *start, const float *d
     r->launches++;
     CUDA_TRY(cudaStreamSynchronize(r->stream));
     CUDA_TRY(cudaMemcpy(out, o.p, count * 4ull, cudaMemcpyDeviceToHost));
-    s.release(); d.release(); o.release(); n.release();
     return S3R_OK;
 }
 
@@ -1182,7 +1168,6 @@ extern "C" int s3r_debug_exact_math(S3RRenderer *r, uint32_t mode, uint64_t firs
     r->launches++;
     CUDA_TRY(cudaStreamSynchronize(r->stream));
     CUDA_TRY(cudaMemcpy(result, res.p, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    res.release();
     return S3R_OK;
 }
 
@@ -1227,7 +1212,6 @@ extern "C" int s3r_set_option(S3RRenderer *r, const char *name, int64_t value) {
         cudaStreamSynchronize(r->stream); r->opt_clusters = (int)value; return S3R_OK;
     }
     if (!strcmp(name, "cluster_cull")) { r->opt_cluster_cull = value != 0; return S3R_OK; }
-    if (!strcmp(name, "dependent_launch")) { set_dependent_launch(value != 0); return S3R_OK; }   // (process-wide)
     if (!strcmp(name, "tensor_store")) { r->opt_tmap = value != 0; return S3R_OK; }
     if (!strcmp(name, "flat_max")) {   // >= 16: the record-free direct walk handles boxes under 16 x 16 whatever this says
         if (value < 16 || value > 65536) { return fail(S3R_E_ARG, "flat_max out of range"); }
@@ -1242,7 +1226,7 @@ extern "C" int s3r_set_option(S3RRenderer *r, const char *name, int64_t value) {
         return S3R_OK;
     }
     if (!strcmp(name, "timing")) { r->opt_timing = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 20)); r->timing_phase = 0; return S3R_OK; }
-    if (!strcmp(name, "pin_host")) { r->opt_pin_host = value != 0; if (!value) { unpin_all(r); } return S3R_OK; }
+    if (!strcmp(name, "pin_host")) { r->opt_pin_host = value != 0; if (!value) { r->pins.clear(); } return S3R_OK; }
     if (!strcmp(name, "views_per_chunk")) {
         if (value < 1) { return fail(S3R_E_ARG, "views_per_chunk < 1"); }
         r->views_per_chunk = (uint32_t)value;
@@ -1250,9 +1234,8 @@ extern "C" int s3r_set_option(S3RRenderer *r, const char *name, int64_t value) {
     }
     if (!strcmp(name, "setup_capacity")) {  // test hook: force the regrow path
         if (value < 1) { return fail(S3R_E_ARG, "setup_capacity < 1"); }
-        cudaStreamSynchronize(r->stream);
-        r->setup_cap = (uint32_t)value; r->tile_cap = 4; r->big_cap = 4; r->walk_cap = 8; r->walk_q.release();
-        r->vis.release(); r->shade.release(); r->head.release(); r->slot_of.release(); r->entries.release(); r->big_list.release(); r->rowbase.release();
+        FrameScratch &b = r->scratch;
+        b.setup_cap = (uint32_t)value; b.tile_cap = 4; b.big_cap = 4; b.walk_cap = 8;
         return S3R_OK;
     }
     if (!strcmp(name, "rowtab_capacity")) {   // test hook: row-start table size in floats per view (0: empty, < 0: default)
@@ -1297,7 +1280,7 @@ struct MultiGpu {
     bool stop = false;
     MultiJob job{};
     int pin = 1, bands = 4;   // bands: raster / shading launches per GPU and frame, each followed by its rows' copy
-    std::vector<HostPin> pins;
+    HostPins pins{cudaHostRegisterPortable};
     // S3R_MULTI_TRACE=1: where a frame's wall time goes (microseconds, summed; printed every 256 frames to stderr)
     int trace = 0;
     uint64_t traced = 0;
@@ -1342,7 +1325,6 @@ int multi_worker_frame(MultiGpu *mg, int k) {
         const uint32_t last_y = ((owned - 1u) * n + (uint32_t)k) * TILE_H, last_rows = std::min<uint32_t>(TILE_H, j.H - last_y);
         uint8_t *dst0 = j.pinned ? reinterpret_cast<uint8_t *>(j.host_out + (size_t)k * TILE_H * j.W) : me.staging;
         const size_t dpitch = j.pinned ? tile_bytes * n : tile_bytes;
-        uint32_t band_rows[S3RRenderer::MAX_SLICES] = {};
         uint32_t done_tiles = 0;
         MultiGpu::Trace *tr = mg->trace ? &mg->tr[(size_t)k] : nullptr;
         int n_bands = 0;
@@ -1350,8 +1332,8 @@ int multi_worker_frame(MultiGpu *mg, int k) {
             if (!tr->e0) { cudaEventCreate(&tr->e0); for (int b = 0; b < 16; b++) { cudaEventCreate(&tr->eb[b]); cudaEventCreate(&tr->ee[b]); } }
             CUDA_TRY(cudaEventRecord(tr->e0, r->stream));
         }
-        const std::function<int(int)> copy_band = [&](int b) -> int {
-            const uint32_t upto = std::min(owned, (band_rows[b] + TILE_H - 1u) / TILE_H);   // owned tile rows finished after band b
+        const BandFn copy_band = [&](int b, uint32_t end_row) -> int {
+            const uint32_t upto = std::min(owned, (end_row + TILE_H - 1u) / TILE_H);   // owned tile rows finished after band b
             CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, r->ev_raster[b], 0));
             if (tr && b < 16) { CUDA_TRY(cudaEventRecord(tr->eb[b], r->copy_stream)); n_bands = b + 1; }
             const uint32_t full_end = (upto == owned && last_rows != (uint32_t)TILE_H) ? owned - 1u : upto;
@@ -1367,7 +1349,7 @@ int multi_worker_frame(MultiGpu *mg, int k) {
             if (tr && b < 16) { CUDA_TRY(cudaEventRecord(tr->ee[b], r->copy_stream)); }
             return S3R_OK;
         };
-        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, r->frame.p, r->stream, mg->bands, band_rows, false, n, (uint32_t)k, &copy_band);
+        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, r->frame.p, r->stream, mg->bands, false, copy_band);
         if (rc) { return rc; }
         r->last_views = 1; r->last_W = j.W; r->last_H = j.H; r->last_stream = r->stream;
         const auto t_launched = std::chrono::steady_clock::now();
@@ -1421,27 +1403,13 @@ void multi_worker(MultiGpu *mg, int k) {
     }
 }
 
-bool multi_pin(MultiGpu *mg, const void *ptr, size_t bytes) {
-    if (!mg->pin) { return false; }
-    for (auto &p : mg->pins) { if (p.ptr == ptr && p.bytes >= bytes) { return true; } }
-    for (size_t i = 0; i < mg->pins.size();) {   // a new buffer (or a resize): drop registrations that overlap it
-        const char *a = static_cast<const char *>(mg->pins[i].ptr), *b = static_cast<const char *>(ptr);
-        if (a < b + bytes && b < a + mg->pins[i].bytes) { cudaHostUnregister(const_cast<void *>(mg->pins[i].ptr)); mg->pins.erase(mg->pins.begin() + (long)i); }
-        else { i++; }
-    }
-    if (mg->pins.size() >= 8) { for (auto &p : mg->pins) { cudaHostUnregister(const_cast<void *>(p.ptr)); } mg->pins.clear(); }
-    if (cudaHostRegister(const_cast<void *>(ptr), bytes, cudaHostRegisterPortable) != cudaSuccess) { cudaGetLastError(); return false; }
-    mg->pins.push_back(HostPin{ptr, bytes});
-    return true;
-}
-
 int multi_render(MultiGpu *mg, const float *matrix, float factor, uint32_t W, uint32_t H, uint32_t *host_out) {
     if (W == 0 || H == 0 || W > 65535 || H > 65535) { return fail(S3R_E_ARG, "bad frame geometry"); }
     const size_t px = (size_t)W * H;
     const auto t_call = std::chrono::steady_clock::now();
     for (int pass = 0; pass < 2; pass++) {
         cudaSetDevice(mg->w[0].r->device);
-        const bool pinned = pass == 0 && multi_pin(mg, host_out, px * 4);
+        const bool pinned = pass == 0 && mg->pin && mg->pins.pin(host_out, px * 4);
         if (pinned) { plant_sentinels(host_out, px); }
         mg->job = MultiJob{matrix, factor, W, H, host_out, pinned};
         if (mg->trace) { mg->us_pin += us_since(t_call); mg->t_publish = std::chrono::steady_clock::now(); }
@@ -1482,7 +1450,6 @@ int multi_render(MultiGpu *mg, const float *matrix, float factor, uint32_t W, ui
             return S3R_OK;
         }
         // the DMA went to pages the CPU no longer sees (a registration outlived its allocation): drop every pin, go again through staging
-        for (auto &p : mg->pins) { cudaHostUnregister(const_cast<void *>(p.ptr)); }
         mg->pins.clear();
         mg->pin = 0;
     }
@@ -1578,11 +1545,10 @@ extern "C" void s3r_dropin_reset(void) {
 extern "C" void s3r_dropin_release_pins(void) {
     if (g_multi) {
         cudaSetDevice(g_multi->w[0].r->device);
-        for (auto &p : g_multi->pins) { cudaHostUnregister(const_cast<void *>(p.ptr)); }
         g_multi->pins.clear();
     } else if (g_renderer) {
         cudaSetDevice(g_renderer->device);
-        unpin_all(g_renderer);
+        g_renderer->pins.clear();
     }
 }
 
