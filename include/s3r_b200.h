@@ -153,7 +153,8 @@ S3R_API int s3r_set_option(S3RRenderer *r, const char *name, int64_t value);
 /* options: "tma_store" (1 = cp.async.bulk tile write-out, default; 0 = plain stores),
  *          "pin_host" (1 = cudaHostRegister the caller's frame buffers; default 0 — only for callers that
  *                      keep the buffer mapped while they pass it; drop-in: env S3R_PIN_HOST=1),
- *          "views_per_chunk" (views per kernel launch set, default 256), "timing" (per-stage and per-kernel events, default 0
+ *          "views_per_chunk" (views per kernel launch set, 1..65535, default 256: a chunk's views are a grid dimension of
+ *          its launches), "timing" (per-stage and per-kernel events, default 0
  *          = off; n > 1: on every n-th submission only),
  *          "fused_small" (1 = one fused geometry CTA per view for scenes of at most 1920 triangles, default),
  *          "direct_small" (general path: 1 = small unclipped survivors are walked by the classify kernel without a setup

@@ -1228,7 +1228,8 @@ extern "C" int s3r_set_option(S3RRenderer *r, const char *name, int64_t value) {
     if (!strcmp(name, "timing")) { r->opt_timing = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 20)); r->timing_phase = 0; return S3R_OK; }
     if (!strcmp(name, "pin_host")) { r->opt_pin_host = value != 0; if (!value) { r->pins.clear(); } return S3R_OK; }
     if (!strcmp(name, "views_per_chunk")) {
-        if (value < 1) { return fail(S3R_E_ARG, "views_per_chunk < 1"); }
+        // a chunk's views are a grid dimension (y or z) of the per-view kernels, which CUDA limits to 65535
+        if (value < 1 || value > 65535) { return fail(S3R_E_ARG, "views_per_chunk out of range 1..65535"); }
         r->views_per_chunk = (uint32_t)value;
         return S3R_OK;
     }

@@ -19,7 +19,7 @@ static uint32_t rnd() {
     return (uint32_t)(rng_state >> 16);
 }
 
-// mode 0: barycentric-like (s in [-2,2], |d| ~ 1/extent); mode 1: random bit patterns with nearby
+// mode 0: barycentric-like (s in [-2,2], |d| ~ 1/extent, extents up to 4000 or, for walks over 4096, 65535); mode 1: random bit patterns with nearby
 // exponents; mode 2: ties (d = (k + 1/2) ulp(s)); mode 3: subnormal / tiny; mode 4: binade edges with sparse deltas; returns mismatches.
 uint64_t walk_fuzz(uint32_t mode, uint64_t trials, uint32_t max_n, uint64_t seed, float *bad) {
     rng_state = seed * 0x9E3779B97F4A7C15ull + 12345;
@@ -29,7 +29,7 @@ uint64_t walk_fuzz(uint32_t mode, uint64_t trials, uint32_t max_n, uint64_t seed
         uint32_t n = 1 + rnd() % max_n;
         if (mode == 0) {
             s = ((int32_t)rnd() / 2147483648.0f) * 2.0f;
-            float ext = 1.0f + (rnd() % 4000);
+            float ext = 1.0f + (rnd() % (max_n > 4096 ? 65535u : 4000u));   // box extents up to the longest walk
             d = ((int32_t)rnd() / 2147483648.0f) * 3.0f / ext;
         } else if (mode == 1) {
             uint32_t e = 100 + rnd() % 56;

@@ -292,21 +292,31 @@ def test_overflowing_bins_are_regrown(renderer_lib, oracle_port):
 
 
 def test_device_walk_jump_equals_sequential_adds(gpu_renderer, oracle_port):
-    """The device build of walk_jump (division-free path) against true sequential binary32 adds."""
+    """The device build of walk_jump (division-free path) against true sequential binary32 adds, up to the longest jump
+    a frame of 65535 pixels asks for (65534 steps, deltas down to about 1/65535)."""
     rs = np.random.RandomState(11)
     n = 20000
     s = rs.uniform(-2, 2, n).astype(np.float32)
-    d = (rs.uniform(-3, 3, n) / rs.randint(1, 4000, n)).astype(np.float32)
-    k = rs.randint(0, 3841, n).astype(np.uint32)
-    # adversarial: ties, binade floors, zero crossings, stuck walks
-    s[:8] = [2.0030441, 1.0, 1.0, 1.0, 0.0, -1.0, 16777216.0, 0.5]
-    d[:8] = [-3.4061623e-06, 2.0 ** -24, -(2.0 ** -25), 1.5 * 2.0 ** -23, 1e-3, 1e-3, 1.0, 0.0]
-    k[:8] = [1845, 3840, 3840, 3840, 3840, 3840, 100, 77]
+    d = (rs.uniform(-3, 3, n) / rs.randint(1, 65536, n)).astype(np.float32)
+    k = rs.randint(0, 65535, n).astype(np.uint32)
+    # adversarial: ties, binade floors, zero crossings, stuck walks; the same kinds again at 65534 steps
+    adv = [(2.0030441, -3.4061623e-06, 1845), (1.0, 2.0 ** -24, 3840), (1.0, -(2.0 ** -25), 3840), (1.0, 1.5 * 2.0 ** -23, 3840),
+           (0.0, 1e-3, 3840), (-1.0, 1e-3, 3840), (16777216.0, 1.0, 100), (0.5, 0.0, 77),
+           (1.0, 2.0 ** -24, 65534), (1.0, -(2.0 ** -25), 65534), (1.0, 1.5 * 2.0 ** -23, 65534),   # tie binades
+           (1.0 + 65534 * 2.0 ** -23, -(2.0 ** -23), 65534),        # lands exactly on the binade floor at the last step
+           (2.0 + 100 * 2.0 ** -22, -(2.0 ** -22), 65534),          # crosses a binade floor, then walks the finer binade
+           (0.3, -1e-5, 65534), (-0.3, 1e-5, 65534), (0.0, -3.0 / 65535, 65534),   # zero crossings, a walk from zero
+           (1.0, 1.0 / 65535, 65534), (-2.0, 3.0 / 65534, 65534)]
+    for i, (a, b, c) in enumerate(adv):
+        s[i], d[i], k[i] = a, b, c
     got = gpu_renderer.debug_walk(s, d, k)
-    want = s.copy()
+    order = np.argsort(-k.astype(np.int64), kind="stable")   # longest walks first: walk i is live while step < k[i]
+    want, dd, kk = s[order].copy(), d[order], k[order]
+    live = np.searchsorted(-kk.astype(np.int64), -np.arange(int(k.max()), dtype=np.int64), side="left")
     for step in range(int(k.max())):  # vectorised sequential adds in binary32
-        live = k > step
-        want[live] = (want[live] + d[live]).astype(np.float32)
+        m = live[step]
+        want[:m] = want[:m] + dd[:m]
+    want = want[np.argsort(order)]
     assert np.array_equal(got.view(np.uint32), want.view(np.uint32)), int((got.view(np.uint32) != want.view(np.uint32)).sum())
 
 

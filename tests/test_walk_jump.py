@@ -25,10 +25,11 @@ def walk_lib(tmp_path_factory):
 
 
 @pytest.mark.parametrize("mode", [0, 1, 2, 3, 4])
-@pytest.mark.parametrize("max_n", [8, 64, 4096])
+@pytest.mark.parametrize("max_n", [8, 64, 4096, 65536])
 def test_fuzz_against_sequential_adds(walk_lib, mode, max_n):
+    """65536: the longest walks of frames up to 65535 pixels (fewer trials: the loop it is checked against is long)."""
     bad = np.zeros(5, np.float32)
-    trials = 400000 if max_n < 4096 else 150000
+    trials = 400000 if max_n < 4096 else 150000 if max_n == 4096 else 12000
     mism = walk_lib.walk_fuzz(mode, trials, max_n, 1000 + 10 * mode + max_n, bad.ctypes.data)
     assert mism == 0, f"first mismatch (s, d, n, jump, seq) = {bad.tolist()}"
 
