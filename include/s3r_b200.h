@@ -104,6 +104,21 @@ S3R_API float s3r_factor(uint32_t height);   /* near * H / (2 * scale), render-c
  */
 S3R_API int s3r_render_device(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width, uint32_t height,
                       uint32_t y0, uint32_t y1, uint32_t *dev_out, void *stream);
+/* Supersampled anti-aliasing: k x k samples per output pixel, k = samples_per_axis in {1, 2, 4} (anything else, or
+ * k * width or k * height over 65535, returns S3R_E_ARG).  width, height, y0, y1 and the output layout are in OUTPUT pixels,
+ * exactly as for s3r_render_device / s3r_render_host; streams, view chunks, s3r_finish and capacity regrowth behave the same.
+ * Definition: with F the frame s3r_render_device renders at k*width x k*height with the same camera (so s3r_factor(k*height),
+ * half_w = k*width / 2, ... follow from that size), output pixel (x, y), channel c, is
+ *     (sum over i, j < k of F[k*y + j][k*x + i].c  +  k*k / 2) >> log2(k*k)
+ * — a box filter on the stored 8-bit values, rounding half up, no gamma conversion, top byte 0.  The band [y0, y1) renders
+ * rows [k*y0, k*y1) of F.  Consequence: the k samples of an output pixel lie at offsets 0, 1/k, ..., (k-1)/k from its 1x
+ * sample point, so the resolved image is shifted by (k-1)/(2k) pixel against the 1x frame (kept: a moved sample grid would
+ * lose exact parity with the reference's frame).  The k x k samples are resolved on chip; only output pixels reach memory,
+ * but visibility scratch is sized for F: at 3840 x 2160 with k = 4 the key plane is 1.06 GB and the tile kernel's weight
+ * state 3.2 GB per view.  k = 1 is the plain call.  After a render with k > 1, s3r_get_stats, s3r_dump_setups and
+ * s3r_dump_raster_vertices describe F.  Not available with peer frames set (S3R_E_ARG), nor for interleaved rows. */
+S3R_API int s3r_render_device_ssaa(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width, uint32_t height,
+                                   uint32_t y0, uint32_t y1, uint32_t samples_per_axis, uint32_t *dev_out, void *stream);
 /* Interleaved partition for multi-GPU load balance: renders the tile rows a (s3r_tile_height() pixel rows
  * each, counted from the top of the frame) with a % row_stride == row_phase.  Output: those tile rows
  * compacted in order — ceil((ceil(H / th) - row_phase) / row_stride) * th rows of `width` uint32 per view
@@ -133,6 +148,9 @@ S3R_API int s3r_copy_from_device(S3RRenderer *r, void *host_dst, const void *dev
 S3R_API int s3r_finish(S3RRenderer *r);
 S3R_API int s3r_render_host(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width, uint32_t height,
                     uint32_t y0, uint32_t y1, uint32_t *host_out);
+/* s3r_render_host with k x k supersampling: see s3r_render_device_ssaa. */
+S3R_API int s3r_render_host_ssaa(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width, uint32_t height,
+                                 uint32_t y0, uint32_t y1, uint32_t samples_per_axis, uint32_t *host_out);
 
 /* ---- introspection (tests, bench) -------------------------------------------------------- */
 S3R_API int s3r_get_stats(S3RRenderer *r, uint32_t view, S3RStats *out);

@@ -1464,6 +1464,9 @@ __device__ __forceinline__ uint32_t shade_pixel(const Frame &f, uint32_t view, u
     return shade_math(f, rz0, rz1, rz2, s, w0, w1, w2);
 }
 
+constexpr uint32_t TILE_W_LOG2 = 6;
+static_assert((1 << TILE_W_LOG2) == TILE_W && TILE_H % 4 == 0, "supersampling: k = 2 and 4 divide the tile, a resolved tile row is whole groups of 4 pixels (24-bit packing)");
+
 __device__ __forceinline__ uint32_t swizzled(uint32_t row, uint32_t seg, uint32_t j) {
     return row * TILE_W + seg * SEG + (j ^ (seg & 7u));  // spreads a thread's 8-pixel run over the 16-byte bank groups
 }
@@ -1488,18 +1491,33 @@ __device__ __forceinline__ void tensor_store_tile(const Frame &f, const void *ti
     }
 }
 
+// Box resolve of one k x k block of 0x00RRGGBB samples (k = 1 << l, l = 1 or 2) whose rows lie `pitch` words apart: per
+// channel (sum + k * k / 2) >> log2(k * k), on the stored 8-bit values.  A sum of 16 bytes fits 12 bits, so red and blue
+// share one accumulator.
+__device__ __forceinline__ uint32_t box_resolve(const uint32_t *s, uint32_t pitch, uint32_t l) {
+    const uint32_t k = 1u << l, sh = 2u * l, half = 1u << (sh - 1u);
+    uint32_t rb = 0u, g = 0u;
+    for (uint32_t j = 0; j < k; j++) {
+        for (uint32_t i = 0; i < k; i++) { const uint32_t c = s[j * pitch + i]; rb += c & 0x00FF00FFu; g += c & 0x0000FF00u; }
+    }
+    return (((rb + half * 0x00010001u) >> sh) & 0x00FF00FFu) | (((g + (half << 8)) >> sh) & 0x0000FF00u);
+}
+
 // Write-out of a finished tile whose rows lie in shared memory `pitch` bytes apart, `bpp` bytes per pixel (4: 32-bit pixels,
 // 3: packed 24-bit transport).  One TMA tensor store for the tile (its map counts bytes for the packed format, pixels
 // otherwise), else one bulk copy per row, else plain stores — 32-bit ones, or bytes for packed rows, which are not word
-// aligned in the output.  All threads call.
+// aligned in the output.  All threads call.  tx0, ty0 are the tile's origin in the rendered frame; a supersampled frame's
+// tile holds its (TILE_W x TILE_H) >> ss_log2 resolved output pixels, which go to output coordinates (tile origins and band
+// edges are multiples of k, so every conversion is exact).
 __device__ __forceinline__ void write_tile(const Frame &f, uint32_t view, uint32_t tx0, uint32_t ty0, uint32_t tile_a,
                                            const void *tile, uint32_t pitch, uint32_t bpp) {
     const uint32_t tid = threadIdx.x, unit = bpp == 4u ? 4u : 1u;   // unit: bytes per plain store and per tensor-map element
-    const uint32_t row_bytes = min((uint32_t)TILE_W, f.W - tx0) * bpp;
+    const uint32_t l = f.ss_log2, ow = f.W >> l, ox0 = tx0 >> l;     // output width and the tile's first output column
+    const uint32_t row_bytes = min((uint32_t)TILE_W >> l, ow - ox0) * bpp;
     uint8_t *out = reinterpret_cast<uint8_t *>(f.out) + (size_t)view * f.out_view_stride * bpp;
     const uint8_t *src = static_cast<const uint8_t *>(tile);
     if (f.use_tmap) {
-        tensor_store_tile(f, tile, (int32_t)(tx0 * bpp / unit), tile_first_out_row(f, ty0, tile_a), (int32_t)view);
+        tensor_store_tile(f, tile, (int32_t)(ox0 * bpp / unit), tile_first_out_row(f, ty0, tile_a) >> l, (int32_t)view);
     } else if (f.use_tma) {
         // make the generic-proxy writes to the tile visible to the async (TMA) proxy
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -1507,12 +1525,13 @@ __device__ __forceinline__ void write_tile(const Frame &f, uint32_t view, uint32
         // the bulk copy takes uniform operands, so a warp issues its lanes' copies one after the other: four rows per
         // warp on all eight warps instead of 32 rows on one
         constexpr uint32_t ROWS_PER_WARP = TILE_H / (RASTER_THREADS / 32);
-        static_assert(ROWS_PER_WARP * (RASTER_THREADS / 32) == TILE_H, "tile rows split evenly over the warps");
-        const uint32_t srow = (tid >> 5) * ROWS_PER_WARP + (tid & 31u);
-        if ((tid & 31u) < ROWS_PER_WARP) {
-            const uint32_t yy = ty0 + srow;
+        static_assert(ROWS_PER_WARP * (RASTER_THREADS / 32) == TILE_H && (ROWS_PER_WARP >> 2) > 0u, "tile rows split evenly over the warps");
+        const uint32_t rows_per_warp = ROWS_PER_WARP >> l;
+        const uint32_t srow = (tid >> 5) * rows_per_warp + (tid & 31u);
+        if ((tid & 31u) < rows_per_warp) {
+            const uint32_t yy = ty0 + (srow << l);   // first rendered row of output row srow
             if (yy >= f.y0 && yy < f.y1) {
-                uint8_t *dst = out + (out_row(f, yy, tile_a) * f.W + tx0) * bpp;
+                uint8_t *dst = out + ((out_row(f, yy, tile_a) >> l) * ow + ox0) * bpp;
                 const uint32_t s = (uint32_t)__cvta_generic_to_shared(src + srow * pitch);
                 asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" :: "l"(dst), "r"(s), "r"(row_bytes) : "memory");
             }
@@ -1521,11 +1540,11 @@ __device__ __forceinline__ void write_tile(const Frame &f, uint32_t view, uint32
         }
     } else {
         __syncthreads();
-        const uint32_t per_row = TILE_W * bpp / unit;
-        for (uint32_t i = tid; i < TILE_H * per_row; i += RASTER_THREADS) {
-            const uint32_t pr = i / per_row, off = (i % per_row) * unit, yy = ty0 + pr;
+        const uint32_t per_row = (TILE_W >> l) * bpp / unit;
+        for (uint32_t i = tid; i < (TILE_H >> l) * per_row; i += RASTER_THREADS) {
+            const uint32_t pr = i / per_row, off = (i % per_row) * unit, yy = ty0 + (pr << l);
             if (off < row_bytes && yy >= f.y0 && yy < f.y1) {
-                uint8_t *dst = out + (out_row(f, yy, tile_a) * f.W + tx0) * bpp + off;
+                uint8_t *dst = out + ((out_row(f, yy, tile_a) >> l) * ow + ox0) * bpp + off;
                 if (unit == 4u) { *reinterpret_cast<uint32_t *>(dst) = *reinterpret_cast<const uint32_t *>(src + pr * pitch + off); }
                 else { *dst = src[pr * pitch + off]; }
             }
@@ -1760,7 +1779,7 @@ __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh
                     // tile's list may be shared by several CTAs) overwrites them in any order; shading checks the tags and
                     // falls back to the exact jump on any mismatch.
                     if (atomicMax(krow + KEY_STEP * x, key) < key) {
-                        unsigned long long *ps = f.pstate + 3u * ((size_t)view * f.out_view_stride + orow * f.W + x);
+                        unsigned long long *ps = f.pstate + 3u * ((size_t)view * f.pix_view_stride + orow * f.W + x);
                         const unsigned long long tag = (unsigned long long)win[j] << 32;
                         ps[0] = tag | __float_as_uint(bw0[j]); ps[1] = tag | __float_as_uint(bw1[j]); ps[2] = tag | __float_as_uint(bw2[j]);
                     }
@@ -1818,23 +1837,33 @@ __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh
     }   // tile with triangles
 
     // ---- write-out -------------------------------------------------------------------------
-    if (f.out_packed24) {
-        // host transport format: 3 bytes per pixel.  Pack each row of 64 pixels into 48 words (reusing the dead per-pixel
-        // state), then write out 192-byte rows.
+    // A supersampled frame's tile is resolved first, each k x k block of the colour tile into one output pixel of the dead
+    // per-pixel state, so that only the (TILE_W x TILE_H) >> ss_log2 output pixels leave the SM.
+    const uint32_t l = f.ss_log2, tw_log2 = TILE_W_LOG2 - l;      // output pixels per tile row: 1 << tw_log2
+    uint32_t *res = &sh.k.colour[0][0], *spare = reinterpret_cast<uint32_t *>(sh.u.state);
+    if (l) {
         __syncthreads();
-        constexpr uint32_t PW = TILE_W * 3u / 4u;                       // packed words per tile row
-        uint32_t *packed = reinterpret_cast<uint32_t *>(sh.u.state);   // [TILE_H][PW]
-        for (uint32_t g = tid; g < TILE_H * (TILE_W / 4); g += RASTER_THREADS) {
-            const uint32_t pr = g / (TILE_W / 4), q = g % (TILE_W / 4);
-            const uint4 p = *reinterpret_cast<const uint4 *>(&sh.k.colour[pr][q * 4]);
-            uint32_t *o = packed + pr * PW + q * 3u;
+        for (uint32_t i = tid; i < (uint32_t)(TILE_W * TILE_H) >> (2u * l); i += RASTER_THREADS) {
+            spare[i] = box_resolve(&sh.k.colour[(i >> tw_log2) << l][(i & ((1u << tw_log2) - 1u)) << l], TILE_W, l);
+        }
+        uint32_t *const t = res; res = spare; spare = t;
+    }
+    if (f.out_packed24) {
+        // host transport format: 3 bytes per pixel.  Pack each row of 64 (supersampled: 64 / k) pixels into 3/4 as many
+        // words (into the other buffer), then write out the rows.
+        __syncthreads();
+        const uint32_t pw = (3u << tw_log2) / 4u;   // packed words per tile row
+        for (uint32_t g = tid; g < (uint32_t)(TILE_H * TILE_W / 4) >> (2u * l); g += RASTER_THREADS) {
+            const uint32_t pr = g >> (tw_log2 - 2u), q = g & ((1u << (tw_log2 - 2u)) - 1u);
+            const uint4 p = *reinterpret_cast<const uint4 *>(res + (pr << tw_log2) + q * 4u);
+            uint32_t *o = spare + pr * pw + q * 3u;
             o[0] = p.x | (p.y << 24);
             o[1] = (p.y >> 8) | (p.z << 16);
             o[2] = (p.z >> 16) | (p.w << 8);
         }
-        write_tile(f, view, tx0, ty0, tile_a, packed, PW * 4u, 3u);
+        write_tile(f, view, tx0, ty0, tile_a, spare, pw * 4u, 3u);
     } else {
-        write_tile(f, view, tx0, ty0, tile_a, &sh.k.colour[0][0], TILE_W * 4u, 4u);
+        write_tile(f, view, tx0, ty0, tile_a, res, 4u << tw_log2, 4u);
     }
 }
 
@@ -2039,7 +2068,7 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
     const uint32_t bx0 = blockIdx.x * SHADE_B, br0 = blockIdx.y * SHADE_BH;       // block origin: pixel column, row within [row0, row0 + nrows)
     const bool broken = f.counters[view * C_COUNT + C_OVERFLOW] != 0;            // incomplete lists: the host renders the frame again
     if (tid == 0) { sh.count = 0; sh.n_tri = 0; }
-    const size_t vbase = (size_t)view * f.out_view_stride;
+    const size_t vbase = (size_t)view * f.pix_view_stride;   // (pstate)
     // ---- 1. keys -> compacted list of covered pixels + distinct triangles ---------------------------
     // A thread reads (and clears) the keys of one column of 4 rows — one 32-byte sector of the key plane where the block
     // starts on a multiple of 4 output rows (always, except in bands that begin inside a tile row).
@@ -2204,15 +2233,30 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
         }
     }
     // ---- 4. write-out: 4 consecutive pixels per thread --------------------------------------------
-    const uint32_t x0 = bx0 + pc;
-    if (br0 + pr >= nrows || x0 >= f.W) { return; }
-    const uint4 c = *reinterpret_cast<const uint4 *>(&sh.colour[pr][pc]);
-    const uint32_t rgb[4] = {c.x, c.y, c.z, c.w};
-    const size_t base = vbase + (size_t)(row0 + br0 + pr) * f.W + x0;
+    // A supersampled frame's block has (SHADE_B x SHADE_BH) >> ss_log2 output pixels: the first threads resolve them from
+    // the colour block, 4 consecutive ones each, and store them at output coordinates (row0, br0 and nrows are multiples
+    // of k, so is W).
+    const uint32_t l = f.ss_log2, w = f.W >> l;
+    uint32_t x0 = bx0 + pc, brow = br0 + pr, rgb[4];   // output column and row (within the band's output rows)
+    if (l == 0u) {
+        if (brow >= nrows || x0 >= f.W) { return; }
+        const uint4 c = *reinterpret_cast<const uint4 *>(&sh.colour[pr][pc]);
+        rgb[0] = c.x; rgb[1] = c.y; rgb[2] = c.z; rgb[3] = c.w;
+    } else {
+        const uint32_t q_log2 = 3u - l;   // output quads per block row: (SHADE_B >> l) / 4
+        static_assert(SHADE_B == 32u && SHADE_BH % 4u == 0u, "supersampling: whole quads of output pixels per block row");
+        if (tid >= (SHADE_PIX >> (2u * l + 2u))) { return; }
+        const uint32_t opr = tid >> q_log2, opc = (tid & ((1u << q_log2) - 1u)) * 4u;
+        x0 = (bx0 >> l) + opc; brow = (br0 >> l) + opr;
+        if (brow >= (nrows >> l) || x0 >= w) { return; }
+#pragma unroll
+        for (int q = 0; q < 4; q++) { rgb[q] = box_resolve(&sh.colour[opr << l][(opc + q) << l], SHADE_B, l); }
+    }
+    const size_t base = (size_t)view * f.out_view_stride + (size_t)((row0 >> l) + brow) * w + x0;
     if (f.n_peers) {
         // fused assembly: this row goes to its absolute place in every rank's frame (one 16-byte store per
         // destination; remote ones travel over NVLink while the CTA's other warps are still shading)
-        const uint32_t py = pixel_y(f, row0 + br0 + pr);
+        const uint32_t py = pixel_y(f, row0 + brow);
         if (py < f.H) {
             const size_t at = ((size_t)view * f.H + py) * f.W + x0;
             const bool wide = x0 + 3u < f.W && (at & 3u) == 0;
@@ -2226,18 +2270,18 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
     }
     if (f.out_packed24) {
         uint8_t *o = reinterpret_cast<uint8_t *>(f.out) + base * 3u;
-        if (x0 + 3u < f.W && (reinterpret_cast<uintptr_t>(o) & 3u) == 0) {
+        if (x0 + 3u < w && (reinterpret_cast<uintptr_t>(o) & 3u) == 0) {
             uint32_t *o32 = reinterpret_cast<uint32_t *>(o);
             o32[0] = rgb[0] | (rgb[1] << 24); o32[1] = (rgb[1] >> 8) | (rgb[2] << 16); o32[2] = (rgb[2] >> 16) | (rgb[3] << 8);
         } else {
-            for (int k = 0; k < 4 && x0 + k < f.W; k++) { o[3 * k] = rgb[k] & 255u; o[3 * k + 1] = (rgb[k] >> 8) & 255u; o[3 * k + 2] = rgb[k] >> 16; }
+            for (int k = 0; k < 4 && x0 + k < w; k++) { o[3 * k] = rgb[k] & 255u; o[3 * k + 1] = (rgb[k] >> 8) & 255u; o[3 * k + 2] = rgb[k] >> 16; }
         }
     } else {
         uint32_t *o = f.out + base;
-        if (x0 + 3u < f.W && (reinterpret_cast<uintptr_t>(o) & 15u) == 0) {
+        if (x0 + 3u < w && (reinterpret_cast<uintptr_t>(o) & 15u) == 0) {
             *reinterpret_cast<uint4 *>(o) = make_uint4(rgb[0], rgb[1], rgb[2], rgb[3]);
         } else {
-            for (int k = 0; k < 4 && x0 + k < f.W; k++) { o[k] = rgb[k]; }
+            for (int k = 0; k < 4 && x0 + k < w; k++) { o[k] = rgb[k]; }
         }
     }
 }

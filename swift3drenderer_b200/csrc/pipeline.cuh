@@ -157,7 +157,12 @@ struct Frame {
     uint32_t *peer_out[MAX_PEERS];
     uint32_t n_peers;
     uint32_t *out;
-    unsigned long long out_view_stride;  // pixels
+    unsigned long long out_view_stride;  // output pixels per view
+    unsigned long long pix_view_stride;  // pixels per view of the frame as rendered (pstate); equals out_view_stride unless ss_log2 > 0
+    // supersampling: the frame above (W x H, rows [y0, y1)) is rendered with k x k samples per output pixel, k = 1 << ss_log2
+    // (0, 1, 2), and every k x k block is box-resolved in the write-out: `out` holds (W >> ss_log2) x ((y1 - y0) >> ss_log2)
+    // pixels per view.  W, H, y0 and y1 are multiples of k; row_stride == 1 and no peer frames when ss_log2 > 0.
+    uint32_t ss_log2;
     int use_tma;
     uint32_t flat_max;  // recorded triangles under flat_max x flat_max pixels are walked flat (post_setup), larger ones by tiles
     int direct_small;   // 1 (general path): small unclipped survivors are walked by the classify kernel and shaded from the raw scene
@@ -173,8 +178,8 @@ struct Frame {
     float *rowtab;          // [views][rowtab_cap]: per triangle a block [component][box row]
     uint32_t *rowbase;      // [views][setup_cap] block offset per survivor slot, NO_TRI = none (flat-walked, or the table was full)
     uint32_t rowtab_cap;
-    // tile_raster write-out as ONE 3-D TMA tensor store per tile (box 64 x 32 x 1 of {x, output row, view}; rows and
-    // columns outside the output are clipped by the hardware) instead of 32 bulk row copies
+    // tile_raster write-out as ONE 3-D TMA tensor store per tile (box (64 x 32) >> ss_log2 x 1 of {x, output row, view}; rows
+    // and columns outside the output are clipped by the hardware) instead of one bulk copy per row
     int use_tmap;
     CUtensorMap out_map;    // 64-byte aligned member of a __grid_constant__ parameter
 };

@@ -600,7 +600,7 @@ static int ensure_scratch(S3RRenderer *r, Frame &f, bool partitioned, bool bande
             CUDA_TRY(b.keys.ensure((size_t)f.n_views * f.key_view_stride + 2));
             CUDA_TRY(cudaMemsetAsync(b.keys.p, 0, b.keys.n * sizeof(unsigned long long), s));
         }
-        CUDA_TRY(b.pstate.ensure(3u * ((size_t)f.n_views * f.out_view_stride + 2)));
+        CUDA_TRY(b.pstate.ensure(3u * ((size_t)f.n_views * f.pix_view_stride + 2)));
         f.pstate = b.pstate.p;
     }
     f.keys = b.keys.p;
@@ -627,9 +627,11 @@ static int ensure_scratch(S3RRenderer *r, Frame &f, bool partitioned, bool bande
 }
 
 // Tensor map of a submission's output for tile_raster's one-store-per-tile write-out: {x, output row, view}, 32-bit
-// pixels or (packed host transport) bytes with 3 per pixel.  cuTensorMapEncodeTiled comes from the driver through the
+// pixels or (packed host transport) bytes with 3 per pixel; W, rows and the box (box_w x box_h pixels: a tile, or a
+// supersampled tile's resolved pixels) in output pixels.  cuTensorMapEncodeTiled comes from the driver through the
 // runtime's entry-point query, so the library does not link libcuda.  false = use the bulk row copies.
-static bool encode_out_map(CUtensorMap *map, void *base, uint32_t W, uint64_t rows, uint32_t views, uint64_t view_stride_px, bool packed24) {
+static bool encode_out_map(CUtensorMap *map, void *base, uint32_t W, uint64_t rows, uint32_t views, uint64_t view_stride_px, bool packed24,
+                           uint32_t box_w, uint32_t box_h) {
     typedef CUresult (*EncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -646,7 +648,7 @@ static bool encode_out_map(CUtensorMap *map, void *base, uint32_t W, uint64_t ro
     const uint64_t bpp = packed24 ? 3 : 4;
     const cuuint64_t dims[3] = {packed24 ? (cuuint64_t)W * 3u : (cuuint64_t)W, rows, views};
     const cuuint64_t strides[2] = {(cuuint64_t)W * bpp, view_stride_px * bpp};   // bytes, dimensions 1 and 2
-    const cuuint32_t box[3] = {packed24 ? (cuuint32_t)TILE_W * 3u : (cuuint32_t)TILE_W, (cuuint32_t)TILE_H, 1u};
+    const cuuint32_t box[3] = {packed24 ? box_w * 3u : box_w, box_h, 1u};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
     if (strides[0] % 16u || strides[1] % 16u) { return false; }
     return encode(map, packed24 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, base, dims, strides, box, estr,
@@ -711,16 +713,18 @@ static void mark_kernel(void *ctx, const char *kernel) {
     if (n < S3RRenderer::MAX_MARKS && cudaEventRecord(m->r->ev_mark[m->slot][n], m->s) == cudaSuccess) { m->r->mark_name[m->slot][n++] = kernel; }
 }
 
-// Called by a host render after band b's raster launch and the record of r->ev_raster[b]; end_row is the first pixel
-// row (relative to y0) after band b.
+// Called by a host render after band b's raster launch and the record of r->ev_raster[b]; end_row is the first output
+// row (relative to the output's first row) after band b.
 typedef std::function<int(int b, uint32_t end_row)> BandFn;
 
 // One submission of n_views views: pixel rows [y0, y1) of the W x H frame, or (row_stride > 1; y0 = 0, y1 = H) the tile
-// rows a with a % row_stride == row_phase, compacted.  The tile rows are rasterised in raster_bands launches; with
-// after_band (host renders), r->ev_raster[b] is recorded after band b and after_band runs.
+// rows a with a % row_stride == row_phase, compacted.  ss_log2 > 0 (row_stride 1 only): W, H, y0, y1 are the supersampled
+// frame's, multiples of k = 1 << ss_log2, and dev_out receives its box-resolved (W / k) x ((y1 - y0) / k) pixels per view.
+// The tile rows are rasterised in raster_bands launches; with after_band (host renders), r->ev_raster[b] is recorded after
+// band b and after_band runs.
 static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
-                        uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, cudaStream_t s, int raster_bands = 1,
-                        bool packed24 = false, const BandFn &after_band = nullptr) {
+                        uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, cudaStream_t s,
+                        int raster_bands = 1, bool packed24 = false, const BandFn &after_band = nullptr) {
     Frame f;
     memset(&f, 0, sizeof(f));
     f.tiles_x = (W + TILE_W - 1) / TILE_W;
@@ -736,8 +740,11 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     f.n_tiles = f.tiles_x * f.tiles_y;
     f.n_views = n_views;
     f.W = W; f.H = H; f.y0 = y0; f.y1 = y1;
-    f.out_view_stride = row_stride == 1 ? (unsigned long long)W * (y1 - y0) : (unsigned long long)W * f.tiles_y * TILE_H;
-    f.key_view_stride = (unsigned long long)W * (((f.out_view_stride / W) + 3u) & ~3ull);   // key plane: columns of 4 output rows
+    f.pix_view_stride = row_stride == 1 ? (unsigned long long)W * (y1 - y0) : (unsigned long long)W * f.tiles_y * TILE_H;
+    f.out_view_stride = f.pix_view_stride >> (2u * ss_log2);
+    f.ss_log2 = ss_log2;
+    const uint32_t out_w = W >> ss_log2;
+    f.key_view_stride = (unsigned long long)W * (((f.pix_view_stride / W) + 3u) & ~3ull);   // key plane: columns of 4 output rows
     const bool partitioned = row_stride > 1 || y0 > 0 || y1 < H;
     int rc = ensure_scratch(r, f, partitioned, raster_bands > 1, s);
     if (rc) { return rc; }
@@ -780,11 +787,12 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     f.n_peers = r->n_peers;
     for (uint32_t k = 0; k < r->n_peers; k++) { f.peer_out[k] = r->peer_out[k]; }
     f.out_packed24 = packed24 ? 1 : 0;
-    f.use_tma = r->opt_tma && (W % (packed24 ? 16 : 4) == 0) && ((reinterpret_cast<uintptr_t>(dev_out) & 15u) == 0);
+    f.use_tma = r->opt_tma && (out_w % (packed24 ? 16 : 4) == 0) && ((reinterpret_cast<uintptr_t>(dev_out) & 15u) == 0);
     // (interleaved tile rows keep the row copies: rows past H stay unwritten; so do bands that start inside a tile row —
     // the store's start coordinate must not be negative)
     if (f.use_tma && r->opt_tmap && f.direct_bin && dev_out && row_stride == 1 && y0 % TILE_H == 0) {
-        f.use_tmap = encode_out_map(&f.out_map, dev_out, W, (uint64_t)(f.out_view_stride / W), n_views, f.out_view_stride, packed24) ? 1 : 0;
+        f.use_tmap = encode_out_map(&f.out_map, dev_out, out_w, (uint64_t)(f.out_view_stride / out_w), n_views, f.out_view_stride, packed24,
+                                    (uint32_t)TILE_W >> ss_log2, (uint32_t)TILE_H >> ss_log2) ? 1 : 0;
     }
     if (timed) { CUDA_TRY(cudaEventRecord(r->ev_t0[slot], s)); }
     if (f.n_peers && (f.direct_bin || packed24)) { return fail(S3R_E_ARG, "peer frames need the general path (scene over 1920 triangles) and device output"); }
@@ -813,7 +821,7 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
             // so that the link starts as early as the GPU allows
             CUDA_TRY(cudaEventRecord(r->ev_raster[b], s));
             const uint32_t end_row = (f.tile_row0 + f.raster_row0 + f.raster_rows) * TILE_H;
-            int rc2 = after_band(b, std::min(y1, std::max(y0, end_row)) - y0);
+            int rc2 = after_band(b, (std::min(y1, std::max(y0, end_row)) - y0) >> ss_log2);   // (band edges are tile rows: exact)
             if (rc2) { return rc2; }
         }
     }
@@ -824,9 +832,10 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
 }
 
 // The device entry points: validation, stream choice and the view-chunk loop.  row_stride == 1: pixel rows [y0, y1);
-// otherwise y0 = 0, y1 = H and the tile rows a with a % row_stride == row_phase.
+// otherwise y0 = 0, y1 = H and the tile rows a with a % row_stride == row_phase.  ss_log2 > 0: the supersampled frame
+// (see render_chunk); W, H, y0, y1 are its own, the output has k x k fewer pixels.
 static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
-                         uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, void *stream) {
+                         uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, void *stream) {
     if (!r || !cams || (!dev_out && r->n_peers == 0)) { return fail(S3R_E_ARG, "null argument"); }
     if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
     if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0 || row_stride == 0 || row_phase >= row_stride) {
@@ -837,10 +846,10 @@ static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, ui
     CUDA_TRY(cudaSetDevice(r->device));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
     r->last_stream = s;
-    const size_t view_px = (size_t)W * (row_stride == 1 ? y1 - y0 : (tile_rows - row_phase + row_stride - 1) / row_stride * TILE_H);
+    const size_t view_px = ((size_t)W * (row_stride == 1 ? y1 - y0 : (tile_rows - row_phase + row_stride - 1) / row_stride * TILE_H)) >> (2u * ss_log2);
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
-        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, dev_out + view_px * v0, s);
+        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, ss_log2, dev_out + view_px * v0, s);
         if (rc) { return rc; }
         r->last_views = nv;
     }
@@ -850,12 +859,33 @@ static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, ui
 
 extern "C" int s3r_render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
                                  uint32_t y0, uint32_t y1, uint32_t *dev_out, void *stream) {
-    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, dev_out, stream);
+    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, 0, dev_out, stream);
+}
+
+// Validation shared by the supersampled entry points: k = samples_per_axis in {1, 2, 4}, the k·W x k·H frame within the
+// ABI's 65535-pixel limit, a band [y0, y1) of the output frame, no peer frames.  *ss_log2 = log2(k).  The band is checked
+// here, in output rows, because the callers scale it by k: an unchecked y0 of 2^31 or more would wrap.
+static int check_ssaa(const S3RRenderer *r, uint32_t k, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1, uint32_t *ss_log2) {
+    if (k != 1 && k != 2 && k != 4) { return fail(S3R_E_ARG, "samples_per_axis must be 1, 2 or 4"); }
+    if ((uint64_t)k * W > 65535 || (uint64_t)k * H > 65535) { return fail(S3R_E_ARG, "samples_per_axis * width and samples_per_axis * height must not exceed 65535"); }
+    if (y0 >= y1 || y1 > H) { return fail(S3R_E_ARG, "bad frame geometry"); }
+    if (r && r->n_peers) { return fail(S3R_E_ARG, "supersampled renders do not assemble peer frames"); }
+    *ss_log2 = k / 2u;   // 1 -> 0, 2 -> 1, 4 -> 2
+    return S3R_OK;
+}
+
+extern "C" int s3r_render_device_ssaa(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0,
+                                      uint32_t y1, uint32_t samples_per_axis, uint32_t *dev_out, void *stream) {
+    uint32_t l = 0;
+    const int rc = check_ssaa(r, samples_per_axis, W, H, y0, y1, &l);
+    if (rc) { return rc; }
+    if (l == 0) { return s3r_render_device(r, cams, n_views, W, H, y0, y1, dev_out, stream); }
+    return render_device(r, cams, n_views, W << l, H << l, y0 << l, y1 << l, 1, 0, l, dev_out, stream);
 }
 
 extern "C" int s3r_render_device_rows(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
                                       uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, void *stream) {
-    return render_device(r, cams, n_views, W, H, 0, H, row_stride, row_phase, dev_out, stream);
+    return render_device(r, cams, n_views, W, H, 0, H, row_stride, row_phase, 0, dev_out, stream);
 }
 
 extern "C" uint32_t s3r_tile_height(void) { return (uint32_t)TILE_H; }
@@ -924,14 +954,17 @@ static int ensure_staging(S3RRenderer *r, size_t bytes) {
     return S3R_OK;
 }
 
-extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
-                               uint32_t y0, uint32_t y1, uint32_t *host_out) {
+// The host entry points.  ss_log2 > 0: W, H, y0, y1 are the supersampled frame's (see render_chunk); the frame scratch, the
+// staging buffer and the caller's buffer hold output pixels.
+static int render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
+                       uint32_t ss_log2, uint32_t *host_out) {
     if (!r || !cams || !host_out) { return fail(S3R_E_ARG, "null argument"); }
     if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
     // SetupVis and the survivor heads pack box bounds in 16 bits: the same limits as s3r_render_device
     if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0) { return fail(S3R_E_ARG, "bad frame geometry"); }
     CUDA_TRY(cudaSetDevice(r->device));
-    const size_t view_px = (size_t)W * (y1 - y0);
+    const uint32_t out_w = W >> ss_log2;
+    const size_t view_px = ((size_t)W * (y1 - y0)) >> (2u * ss_log2);
     // OPT-IN ("pin_host" option / S3R_PIN_HOST=1): cudaHostRegister the caller's frame buffer so the D2H
     // copy runs at full PCIe rate.  Only safe when the caller keeps that allocation mapped for as long
     // as it passes it (the reference's main loop does: one double buffer, re-allocated on resize only,
@@ -960,7 +993,7 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
             uint32_t row = 0;
             // band b's pixels of all nv views; several views have one band, copied in slices of about 4 MB
             const BandFn copy_band = [&](int b, uint32_t end_row) -> int {
-                const size_t pa = (size_t)row * W * nv, pe = (size_t)end_row * W * nv;
+                const size_t pa = (size_t)row * out_w * nv, pe = (size_t)end_row * out_w * nv;
                 row = end_row;
                 CUDA_TRY(cudaStreamWaitEvent(r->copy_stream, r->ev_raster[b], 0));
                 const size_t n_sl = nv == 1 ? 1 : std::min<size_t>(S3RRenderer::MAX_SLICES, std::max<size_t>(1, chunk_bytes >> 22));
@@ -976,7 +1009,7 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
                 }
                 return S3R_OK;
             };
-            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, r->frame.p, r->stream, bands, packed, copy_band);
+            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, ss_log2, r->frame.p, r->stream, bands, packed, copy_band);
             if (rc) { return rc; }
             r->last_views = nv; r->last_W = W; r->last_H = H;
             // ---- drain: as each slice lands in staging the worker threads move it to the caller ----
@@ -1003,6 +1036,20 @@ extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_vie
         if (!rendered) { return fail(S3R_E_CUDA, "frame scratch still overflowing after 8 regrowths"); }
     }
     return S3R_OK;
+}
+
+extern "C" int s3r_render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
+                               uint32_t y0, uint32_t y1, uint32_t *host_out) {
+    return render_host(r, cams, n_views, W, H, y0, y1, 0, host_out);
+}
+
+extern "C" int s3r_render_host_ssaa(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0,
+                                    uint32_t y1, uint32_t samples_per_axis, uint32_t *host_out) {
+    uint32_t l = 0;
+    const int rc = check_ssaa(r, samples_per_axis, W, H, y0, y1, &l);
+    if (rc) { return rc; }
+    if (l == 0) { return s3r_render_host(r, cams, n_views, W, H, y0, y1, host_out); }
+    return render_host(r, cams, n_views, W << l, H << l, y0 << l, y1 << l, l, host_out);
 }
 
 // --------------------------------------------------------------------------------------------------
@@ -1350,7 +1397,7 @@ int multi_worker_frame(MultiGpu *mg, int k) {
             if (tr && b < 16) { CUDA_TRY(cudaEventRecord(tr->ee[b], r->copy_stream)); }
             return S3R_OK;
         };
-        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, r->frame.p, r->stream, mg->bands, false, copy_band);
+        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, 0, r->frame.p, r->stream, mg->bands, false, copy_band);
         if (rc) { return rc; }
         r->last_views = 1; r->last_W = j.W; r->last_H = j.H; r->last_stream = r->stream;
         const auto t_launched = std::chrono::steady_clock::now();

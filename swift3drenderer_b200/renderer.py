@@ -73,6 +73,7 @@ EXPORTS = [
     "s3r_dropin_reset", "s3r_debug_walk", "s3r_debug_exact_math", "s3r_render_device_rows", "s3r_tile_height",
     "s3r_peer_frame_alloc", "s3r_peer_frame_open", "s3r_peer_frame_release", "s3r_set_peer_frames", "s3r_copy_from_device",
     "s3r_sink_open", "s3r_sink_submit", "s3r_sink_close", "s3r_debug_band_edges", "s3r_get_kernel_timing", "s3r_debug_clusters", "s3r_dropin_devices", "s3r_dropin_release_pins",
+    "s3r_render_device_ssaa", "s3r_render_host_ssaa",
 ]
 
 
@@ -127,6 +128,8 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.s3r_render_device.argtypes = [vp, vp, u32, u32, u32, u32, u32, vp, vp]
     lib.s3r_finish.argtypes = [vp]
     lib.s3r_render_host.argtypes = [vp, vp, u32, u32, u32, u32, u32, vp]
+    lib.s3r_render_device_ssaa.argtypes = [vp, vp, u32, u32, u32, u32, u32, u32, vp, vp]
+    lib.s3r_render_host_ssaa.argtypes = [vp, vp, u32, u32, u32, u32, u32, u32, vp]
     lib.s3r_get_stats.argtypes = [vp, u32, ctypes.POINTER(CStats)]
     lib.s3r_dump_raster_vertices.argtypes = [vp, u32, vp, u64]
     lib.s3r_dump_setups.argtypes = [vp, u32, vp, u64, ctypes.POINTER(u64)]
@@ -290,6 +293,29 @@ class Renderer:
         y1 = height if y1 is None else y1
         self._check(self._lib.s3r_render_device(self._h, cams.ctypes.data, cams.shape[0], width, height, y0, y1,
                                                  ctypes.c_void_p(dev_ptr), ctypes.c_void_p(stream)))
+
+    def render_ssaa(self, cameras, width: int, height: int, samples: int, y0: int = 0, y1: Optional[int] = None,
+                    out: Optional[np.ndarray] = None) -> np.ndarray:
+        """``render`` with ``samples`` x ``samples`` samples per pixel (1, 2 or 4), box-resolved: the frame rendered at
+        ``samples * width`` x ``samples * height``, each block averaged per channel with rounding half up.  Sizes and
+        rows are output pixels."""
+        cams = np.ascontiguousarray(cameras, "<f4").reshape(-1, 12)
+        y1 = height if y1 is None else y1
+        n = cams.shape[0]
+        if out is None:
+            out = np.empty((n, max(y1 - y0, 0), width), np.uint32)
+        assert out.dtype == np.uint32 and out.size == n * max(y1 - y0, 0) * width and out.flags.c_contiguous
+        self._check(self._lib.s3r_render_host_ssaa(self._h, cams.ctypes.data, n, width, height, y0, y1, samples,
+                                                   out.ctypes.data))
+        return out
+
+    def render_device_ssaa(self, cameras, width: int, height: int, samples: int, dev_ptr: int, y0: int = 0,
+                           y1: Optional[int] = None, stream: int = 0) -> None:
+        """``render_device`` with ``samples`` x ``samples`` samples per pixel; see ``render_ssaa``."""
+        cams = np.ascontiguousarray(cameras, "<f4").reshape(-1, 12)
+        y1 = height if y1 is None else y1
+        self._check(self._lib.s3r_render_device_ssaa(self._h, cams.ctypes.data, cams.shape[0], width, height, y0, y1,
+                                                      samples, ctypes.c_void_p(dev_ptr), ctypes.c_void_p(stream)))
 
     def render_device_rows(self, cameras, width: int, height: int, row_stride: int, row_phase: int, dev_ptr: int,
                            stream: int = 0) -> None:
