@@ -119,6 +119,23 @@ S3R_API int s3r_render_device(S3RRenderer *r, const float *cameras, uint32_t n_v
  * s3r_dump_raster_vertices describe F.  Not available with peer frames set (S3R_E_ARG), nor for interleaved rows. */
 S3R_API int s3r_render_device_ssaa(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width, uint32_t height,
                                    uint32_t y0, uint32_t y1, uint32_t samples_per_axis, uint32_t *dev_out, void *stream);
+/* Visibility planes: which triangle each pixel shows and at what depth, for picking, depth compositing and deferred passes
+ * driven by a triangle-ID buffer.  Everything works as in s3r_render_device (cameras, bands [y0, y1), view chunks, streams,
+ * s3r_finish and its render-again contract, statistics and dumps).  Each non-null output is DEVICE memory with the colour
+ * output's layout: n_views x (y1 - y0) x width, tightly packed.
+ *   dev_triangle[p]: the scene triangle index t of the triangle that colours pixel p in the reference's frame; its corners
+ *     are vertex_indices[3t .. 3t+2].  A triangle appended by the near-plane clip (render.cpp:239-257) reports the triangle
+ *     it was cut from.  Background: 0xFFFFFFFF.
+ *   dev_depth[p]: the reference's depth-buffer value at p (render.cpp:363-364), the binary32 interpolated 1/z
+ *     (rvz0*w0 + rvz1*w1) + rvz2*w2 of that triangle; linear depth is 1 / dev_depth[p].  Background: +0.0f.
+ *   dev_out: when non-null, the colour frame, bit-identical to s3r_render_device's.  When null, the call is a
+ *     visibility-only render: nothing is shaded and no colour is written.
+ * Any subset of the three outputs may be null, but not all three.  The planes cost two 4-byte stores per pixel and no
+ * extra kernel launch.  S3R_E_ARG (nothing written): all three outputs null, peer frames set, or bad frame geometry as for
+ * s3r_render_device.  Not available for host output, interleaved rows or supersampling. */
+S3R_API int s3r_render_device_visibility(S3RRenderer *r, const float *cameras, uint32_t n_views, uint32_t width,
+                                         uint32_t height, uint32_t y0, uint32_t y1, uint32_t *dev_out,
+                                         uint32_t *dev_triangle, float *dev_depth, void *stream);
 /* Interleaved partition for multi-GPU load balance: renders the tile rows a (s3r_tile_height() pixel rows
  * each, counted from the top of the frame) with a % row_stride == row_phase.  Output: those tile rows
  * compacted in order — ceil((ceil(H / th) - row_phase) / row_stride) * th rows of `width` uint32 per view

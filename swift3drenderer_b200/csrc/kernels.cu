@@ -1476,6 +1476,22 @@ __device__ __forceinline__ int32_t tile_first_out_row(const Frame &f, uint32_t t
     return f.row_stride == 1u ? (int32_t)ty0 - (int32_t)f.y0 : (int32_t)(div_stride(f, tile_a) * TILE_H);
 }
 
+// Visibility planes (Frame::tri_out, depth_out) of output pixel `at`: `order` is the winner's order key — T + parent for a
+// triangle the near-plane clip appended (render.cpp:239-257), which reports its parent — or NO_TRI for background, whose
+// depth is +0.
+__device__ __forceinline__ void store_planes(const Frame &f, size_t at, uint32_t order, float depth) {
+    if (f.tri_out) { f.tri_out[at] = order == NO_TRI ? NO_TRI : (order >= f.T ? order - f.T : order); }
+    if (f.depth_out) { f.depth_out[at] = depth; }
+}
+
+// ... of pixel (pr, pc) of the tile at (tx0, ty0): written for rows inside the band and columns inside the frame only,
+// at the output row write_tile uses.
+__device__ __forceinline__ void store_tile_planes(const Frame &f, uint32_t view, uint32_t tx0, uint32_t ty0, uint32_t tile_a,
+                                                  uint32_t pr, uint32_t pc, uint32_t order, float depth) {
+    const uint32_t yy = ty0 + pr, x = tx0 + pc;
+    if (yy >= f.y0 && yy < f.y1 && x < f.W) { store_planes(f, (size_t)view * f.out_view_stride + out_row(f, yy, tile_a) * f.W + x, order, depth); }
+}
+
 // One TMA tensor store for a whole tile: the box (TILE_W pixels x TILE_H rows, contiguous in shared memory) goes to
 // {x, row, view} of the output tensor; whatever lies outside the tensor (band edges, a partial last tile) is clipped
 // by the copy engine.  Called by all threads after the tile is complete in shared memory; one thread issues it.
@@ -1594,8 +1610,10 @@ __device__ __forceinline__ bool walk_small(const Frame &f, uint32_t view, uint32
 // One tile (TILE_W x TILE_H pixels).  DIRECT (small scenes): the CTA collects the tile's triangles from the survivor
 // list itself, resolves visibility, shades and writes the colour tile.  !DIRECT (general path): the CTA resolves
 // entries [e0, e1) of the tile's bin list — recorded triangles too large for the flat walk — and merges its winners
-// into the visibility buffer with 64-bit atomicMax, so that a long list can be shared by several CTAs.
-template <bool DIRECT>
+// into the visibility buffer with 64-bit atomicMax, so that a long list can be shared by several CTAs.  PLANES (DIRECT
+// only): the lane that owns a pixel in phase 3 also writes its visibility planes; with no colour output (f.out == null)
+// nothing is shaded or written out.
+template <bool DIRECT, bool PLANES>
 __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh, uint32_t view, uint32_t tile_x, uint32_t tile_y,
                                                 uint32_t e0, uint32_t e1) {
     const uint32_t tid = threadIdx.x;
@@ -1645,6 +1663,11 @@ __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh
         // nothing reaches this tile: it is background (render.cpp:282) — straight to the write-out
 #pragma unroll
         for (int j = 0; j < SEG; j++) { sh.k.colour[row][seg * SEG + j] = kBackground; }
+        if (PLANES) {
+            for (uint32_t p = tid; p < (uint32_t)(TILE_W * TILE_H); p += RASTER_THREADS) {
+                store_tile_planes(f, view, tx0, ty0, tile_a, p / TILE_W, p % TILE_W, NO_TRI, 0.f);
+            }
+        }
     } else {
     float depth[SEG], bw0[SEG], bw1[SEG], bw2[SEG];
     uint32_t win[SEG];
@@ -1829,12 +1852,24 @@ __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh
         const uint32_t p = it * RASTER_THREADS + tid, pr = p / TILE_W, pc = p % TILE_W;
         const uint4 st = sh.u.state[swizzled(pr, pc / SEG, pc % SEG)];
         uint32_t rgb = kBackground;
+        if (PLANES) {
+            uint32_t order = NO_TRI;
+            float depth = 0.f;
+            if (st.w != NO_TRI) {   // the winner's depth as phase 1 computed it (render.cpp:363)
+                const SetupVis *vp = f.vis + (size_t)view * f.setup_cap + st.w;
+                depth = (vp->rvz[0] * __uint_as_float(st.x) + vp->rvz[1] * __uint_as_float(st.y)) + vp->rvz[2] * __uint_as_float(st.z);
+                order = f.head[(size_t)view * f.setup_cap + st.w].z;
+            }
+            store_tile_planes(f, view, tx0, ty0, tile_a, pr, pc, order, depth);
+            if (!f.out) { continue; }
+        }
         if (st.w != NO_TRI) {
             rgb = shade_pixel(f, view, st.w, __uint_as_float(st.x), __uint_as_float(st.y), __uint_as_float(st.z));
         }
         sh.k.colour[pr][pc] = rgb;
     }
     }   // tile with triangles
+    if (PLANES && !f.out) { return; }   // visibility only
 
     // ---- write-out -------------------------------------------------------------------------
     // A supersampled frame's tile is resolved first, each k x k block of the colour tile into one output pixel of the dead
@@ -1867,9 +1902,10 @@ __device__ __forceinline__ void raster_one_tile(const Frame &f, RasterShared &sh
     }
 }
 
+template <bool PLANES>
 __global__ void __launch_bounds__(RASTER_THREADS, RASTER_CTAS) tile_raster(const __grid_constant__ Frame f) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    raster_one_tile<true>(f, *reinterpret_cast<RasterShared *>(smem_raw), blockIdx.z, blockIdx.x, blockIdx.y + f.raster_row0, 0u, 0u);
+    raster_one_tile<true, PLANES>(f, *reinterpret_cast<RasterShared *>(smem_raw), blockIdx.z, blockIdx.x, blockIdx.y + f.raster_row0, 0u, 0u);
 }
 
 // General path: persistent CTAs pop (tile, chunk of its bin list) items from the queue post_setup built.  A tile with
@@ -1892,7 +1928,7 @@ __global__ void __launch_bounds__(RASTER_THREADS, QUEUE_CTAS) tile_raster_queue(
         __syncthreads();
         const uint2 item = f.raster_items[(size_t)view * f.items_cap + i];   // {tile, first entry}
         const uint32_t n = min(f.tile_count[view * f.tile_stride + item.x], f.tile_cap);
-        raster_one_tile<false>(f, sh, view, item.x % f.tiles_x, item.x / f.tiles_x, item.y, min(n, item.y + RASTER_CHUNK));
+        raster_one_tile<false, false>(f, sh, view, item.x % f.tiles_x, item.x / f.tiles_x, item.y, min(n, item.y + RASTER_CHUNK));
     }
 }
 
@@ -2059,7 +2095,9 @@ struct ShadeShared {
     uint32_t count, n_tri;
 };
 
-template <bool HAS_RV>
+// PLANES: step 1 also writes the visibility planes from the keys it reads; with no colour output (f.out == null) the block
+// stops after the keys are cleared.
+template <bool HAS_RV, bool PLANES>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const __grid_constant__ Frame f, uint32_t row0, uint32_t nrows) {
     wait_for_predecessor();
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -2075,6 +2113,7 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
     const uint32_t pr = tid >> 3, pc = (tid & 7u) * 4u;   // write-out (step 4): block row pr, columns pc .. pc + 3
     const uint32_t kr = (tid >> 5) * 4u, kc = tid & 31u;   // keys: block rows kr .. kr + 3 of block column kc
     uint32_t ord[4] = {0u, 0u, 0u, 0u}, mask = 0;
+    uint32_t dep[4] = {0u, 0u, 0u, 0u};   // (PLANES) the keys' depth words
     if (bx0 + kc < f.W && br0 + kr < nrows) {
         unsigned long long *plane = f.keys + (size_t)view * f.key_view_stride;
         const size_t r_first = (size_t)row0 + br0 + kr;
@@ -2083,7 +2122,9 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
             const ulonglong2 lo = kp[0], hi = kp[1];
             const unsigned long long key[4] = {lo.x, lo.y, hi.x, hi.y};
 #pragma unroll
-            for (int k = 0; k < 4; k++) { if (key[k] != 0ull) { ord[k] = ~(uint32_t)key[k]; mask |= 1u << k; } }
+            for (int k = 0; k < 4; k++) {
+                if (key[k] != 0ull) { ord[k] = ~(uint32_t)key[k]; mask |= 1u << k; if (PLANES) { dep[k] = (uint32_t)(key[k] >> 32); } }
+            }
             if (mask & 3u) { kp[0] = make_ulonglong2(0ull, 0ull); }
             if (mask & 12u) { kp[1] = make_ulonglong2(0ull, 0ull); }
         } else {
@@ -2092,12 +2133,27 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
                 if (br0 + kr + k < nrows) {
                     unsigned long long *kp = plane + key_at(f, r_first + k, bx0 + kc);
                     const unsigned long long key = *kp;
-                    if (key != 0ull) { *kp = 0ull; ord[k] = ~(uint32_t)key; mask |= 1u << k; }
+                    if (key != 0ull) { *kp = 0ull; ord[k] = ~(uint32_t)key; mask |= 1u << k; if (PLANES) { dep[k] = (uint32_t)(key >> 32); } }
                 }
             }
         }
     }
     if (broken) { mask = 0; }
+    if (PLANES) {
+        // the key already holds the final winner under every routing; the lanes of a warp are 32 neighbouring columns, so
+        // each store instruction covers 128 contiguous bytes of a plane
+        if (bx0 + kc < f.W) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                if (br0 + kr + k < nrows) {
+                    const bool hit = (mask >> k) & 1u;
+                    store_planes(f, (size_t)view * f.out_view_stride + (size_t)(row0 + br0 + kr + k) * f.W + bx0 + kc,
+                                 hit ? ord[k] : NO_TRI, hit ? __uint_as_float(dep[k]) : 0.f);
+                }
+            }
+        }
+        if (!f.out) { return; }   // visibility only: the keys are read and cleared, nothing is shaded
+    }
     *reinterpret_cast<uint4 *>(&sh.colour[pr][pc]) = make_uint4(kBackground, kBackground, kBackground, kBackground);
     const bool any = __syncthreads_or(mask != 0u);
     if (any) {
@@ -2296,10 +2352,12 @@ cudaError_t configure_kernels() {
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) { return e; }
     cudaDeviceGetAttribute(&g_sm_count, cudaDevAttrMultiProcessorCount, dev);
-    e = cudaFuncSetAttribute(tile_raster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RasterShared));
-    if (e != cudaSuccess) { return e; }
-    e = cudaFuncSetAttribute(tile_raster, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) { return e; }
+    for (auto k : {tile_raster<false>, tile_raster<true>}) {
+        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RasterShared));
+        if (e != cudaSuccess) { return e; }
+        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) { return e; }
+    }
     e = cudaFuncSetAttribute(tile_raster_queue, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RasterShared));
     if (e != cudaSuccess) { return e; }
     e = cudaFuncSetAttribute(tile_raster_queue, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -2309,14 +2367,12 @@ cudaError_t configure_kernels() {
     if (e != cudaSuccess) { return e; }
     e = cudaFuncSetAttribute(direct_walk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) { return e; }
-    e = cudaFuncSetAttribute(shade_tiles<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ShadeShared));
-    if (e != cudaSuccess) { return e; }
-    e = cudaFuncSetAttribute(shade_tiles<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) { return e; }
-    e = cudaFuncSetAttribute(shade_tiles<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ShadeShared));
-    if (e != cudaSuccess) { return e; }
-    e = cudaFuncSetAttribute(shade_tiles<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) { return e; }
+    for (auto k : {shade_tiles<true, false>, shade_tiles<false, false>, shade_tiles<true, true>, shade_tiles<false, true>}) {
+        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ShadeShared));
+        if (e != cudaSuccess) { return e; }
+        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) { return e; }
+    }
     return cudaFuncSetAttribute(triangle_classify, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 
@@ -2365,8 +2421,11 @@ int launch_geometry(const Frame &f, cudaStream_t s, const LaunchMarks *m) {
 }
 
 int launch_raster(const Frame &f, cudaStream_t s, const LaunchMarks *m) {
+    // visibility planes requested: the write-out kernels' PLANES instantiations (the plain ones keep their code)
+    const bool planes = f.tri_out || f.depth_out;
     if (f.direct_bin) {
-        tile_raster<<<dim3(f.tiles_x, f.raster_rows, f.n_views), RASTER_THREADS, sizeof(RasterShared), s>>>(f); mark(m, "tile_raster");
+        (planes ? tile_raster<true> : tile_raster<false>)<<<dim3(f.tiles_x, f.raster_rows, f.n_views), RASTER_THREADS, sizeof(RasterShared), s>>>(f);
+        mark(m, "tile_raster");
         return 1;
     }
     // general path: the queue holds every non-empty tile of the submission, so the tile kernel runs once per frame, with
@@ -2386,8 +2445,9 @@ int launch_raster(const Frame &f, cudaStream_t s, const LaunchMarks *m) {
     }
     if (nrows) {
         const dim3 grid(ceil_div(f.W, SHADE_B), ceil_div(nrows, SHADE_BH), f.n_views);
-        if (f.rv) { launch_chain(shade_tiles<true>, grid, dim3(SHADE_THREADS), sizeof(ShadeShared), s, true, f, row0, nrows); }
-        else { launch_chain(shade_tiles<false>, grid, dim3(SHADE_THREADS), sizeof(ShadeShared), s, true, f, row0, nrows); }
+        const auto shade = f.rv ? (planes ? shade_tiles<true, true> : shade_tiles<true, false>)
+                                : (planes ? shade_tiles<false, true> : shade_tiles<false, false>);
+        launch_chain(shade, grid, dim3(SHADE_THREADS), sizeof(ShadeShared), s, true, f, row0, nrows);
         mark(m, "shade_tiles");
         launches++;
     }

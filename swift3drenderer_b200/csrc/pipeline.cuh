@@ -182,6 +182,13 @@ struct Frame {
     // and columns outside the output are clipped by the hardware) instead of one bulk copy per row
     int use_tmap;
     CUtensorMap out_map;    // 64-byte aligned member of a __grid_constant__ parameter
+    // visibility planes (s3r_render_device_visibility: row_stride == 1, ss_log2 == 0, no peer frames), laid out like `out`:
+    // per pixel the scene index of the winning triangle (a triangle the near-plane clip appended reports its parent;
+    // NO_TRI = background) and its interpolated 1/z (+0 = background).  Null = not requested.  Only the PLANES
+    // instantiations of tile_raster and shade_tiles read these; with a plane set, out == null means visibility only:
+    // nothing is shaded and no colour is written.
+    uint32_t *tri_out;
+    float *depth_out;
 };
 
 // Launchers (kernels.cu).  Each returns the number of kernels it enqueued.  `marks` (optional): called after every kernel

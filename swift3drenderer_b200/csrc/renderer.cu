@@ -720,11 +720,13 @@ typedef std::function<int(int b, uint32_t end_row)> BandFn;
 // One submission of n_views views: pixel rows [y0, y1) of the W x H frame, or (row_stride > 1; y0 = 0, y1 = H) the tile
 // rows a with a % row_stride == row_phase, compacted.  ss_log2 > 0 (row_stride 1 only): W, H, y0, y1 are the supersampled
 // frame's, multiples of k = 1 << ss_log2, and dev_out receives its box-resolved (W / k) x ((y1 - y0) / k) pixels per view.
-// The tile rows are rasterised in raster_bands launches; with after_band (host renders), r->ev_raster[b] is recorded after
-// band b and after_band runs.
+// dev_tri, dev_depth (row_stride 1, ss_log2 0, device output only): the visibility planes, laid out like dev_out, which
+// may then be null (visibility only).  The tile rows are rasterised in raster_bands launches; with after_band (host
+// renders), r->ev_raster[b] is recorded after band b and after_band runs.
 static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
-                        uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, cudaStream_t s,
-                        int raster_bands = 1, bool packed24 = false, const BandFn &after_band = nullptr) {
+                        uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, uint32_t *dev_tri,
+                        float *dev_depth, cudaStream_t s, int raster_bands = 1, bool packed24 = false,
+                        const BandFn &after_band = nullptr) {
     Frame f;
     memset(&f, 0, sizeof(f));
     f.tiles_x = (W + TILE_W - 1) / TILE_W;
@@ -784,10 +786,11 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
     f.factor = r->factor_override != 0.f ? r->factor_override : s3r_factor(H);
     f.band_lo = (float)y0; f.band_hi = (float)y1;
     f.out = dev_out;
+    f.tri_out = dev_tri; f.depth_out = dev_depth;
     f.n_peers = r->n_peers;
     for (uint32_t k = 0; k < r->n_peers; k++) { f.peer_out[k] = r->peer_out[k]; }
     f.out_packed24 = packed24 ? 1 : 0;
-    f.use_tma = r->opt_tma && (out_w % (packed24 ? 16 : 4) == 0) && ((reinterpret_cast<uintptr_t>(dev_out) & 15u) == 0);
+    f.use_tma = r->opt_tma && dev_out && (out_w % (packed24 ? 16 : 4) == 0) && ((reinterpret_cast<uintptr_t>(dev_out) & 15u) == 0);
     // (interleaved tile rows keep the row copies: rows past H stay unwritten; so do bands that start inside a tile row —
     // the store's start coordinate must not be negative)
     if (f.use_tma && r->opt_tmap && f.direct_bin && dev_out && row_stride == 1 && y0 % TILE_H == 0) {
@@ -833,10 +836,12 @@ static int render_chunk(S3RRenderer *r, const float *cams, uint32_t n_views, uin
 
 // The device entry points: validation, stream choice and the view-chunk loop.  row_stride == 1: pixel rows [y0, y1);
 // otherwise y0 = 0, y1 = H and the tile rows a with a % row_stride == row_phase.  ss_log2 > 0: the supersampled frame
-// (see render_chunk); W, H, y0, y1 are its own, the output has k x k fewer pixels.
+// (see render_chunk); W, H, y0, y1 are its own, the output has k x k fewer pixels.  dev_tri, dev_depth: the visibility
+// planes (see render_chunk).
 static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H, uint32_t y0, uint32_t y1,
-                         uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, void *stream) {
-    if (!r || !cams || (!dev_out && r->n_peers == 0)) { return fail(S3R_E_ARG, "null argument"); }
+                         uint32_t row_stride, uint32_t row_phase, uint32_t ss_log2, uint32_t *dev_out, uint32_t *dev_tri,
+                         float *dev_depth, void *stream) {
+    if (!r || !cams || (!dev_out && !dev_tri && !dev_depth && r->n_peers == 0)) { return fail(S3R_E_ARG, "null argument"); }
     if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
     if (W == 0 || H == 0 || W > 65535 || H > 65535 || y0 >= y1 || y1 > H || n_views == 0 || row_stride == 0 || row_phase >= row_stride) {
         return fail(S3R_E_ARG, "bad frame geometry");
@@ -849,7 +854,9 @@ static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, ui
     const size_t view_px = ((size_t)W * (row_stride == 1 ? y1 - y0 : (tile_rows - row_phase + row_stride - 1) / row_stride * TILE_H)) >> (2u * ss_log2);
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
-        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, ss_log2, dev_out + view_px * v0, s);
+        const size_t at = view_px * v0;   // (an output not requested stays null)
+        int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, ss_log2, dev_out ? dev_out + at : dev_out,
+                              dev_tri ? dev_tri + at : dev_tri, dev_depth ? dev_depth + at : dev_depth, s);
         if (rc) { return rc; }
         r->last_views = nv;
     }
@@ -859,7 +866,15 @@ static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, ui
 
 extern "C" int s3r_render_device(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
                                  uint32_t y0, uint32_t y1, uint32_t *dev_out, void *stream) {
-    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, 0, dev_out, stream);
+    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, 0, dev_out, nullptr, nullptr, stream);
+}
+
+extern "C" int s3r_render_device_visibility(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
+                                            uint32_t y0, uint32_t y1, uint32_t *dev_out, uint32_t *dev_triangle,
+                                            float *dev_depth, void *stream) {
+    if (!dev_out && !dev_triangle && !dev_depth) { return fail(S3R_E_ARG, "no output: the colour, triangle and depth outputs are all null"); }
+    if (r && r->n_peers) { return fail(S3R_E_ARG, "visibility planes are not assembled into peer frames"); }
+    return render_device(r, cams, n_views, W, H, y0, y1, 1, 0, 0, dev_out, dev_triangle, dev_depth, stream);
 }
 
 // Validation shared by the supersampled entry points: k = samples_per_axis in {1, 2, 4}, the k·W x k·H frame within the
@@ -880,12 +895,12 @@ extern "C" int s3r_render_device_ssaa(S3RRenderer *r, const float *cams, uint32_
     const int rc = check_ssaa(r, samples_per_axis, W, H, y0, y1, &l);
     if (rc) { return rc; }
     if (l == 0) { return s3r_render_device(r, cams, n_views, W, H, y0, y1, dev_out, stream); }
-    return render_device(r, cams, n_views, W << l, H << l, y0 << l, y1 << l, 1, 0, l, dev_out, stream);
+    return render_device(r, cams, n_views, W << l, H << l, y0 << l, y1 << l, 1, 0, l, dev_out, nullptr, nullptr, stream);
 }
 
 extern "C" int s3r_render_device_rows(S3RRenderer *r, const float *cams, uint32_t n_views, uint32_t W, uint32_t H,
                                       uint32_t row_stride, uint32_t row_phase, uint32_t *dev_out, void *stream) {
-    return render_device(r, cams, n_views, W, H, 0, H, row_stride, row_phase, 0, dev_out, stream);
+    return render_device(r, cams, n_views, W, H, 0, H, row_stride, row_phase, 0, dev_out, nullptr, nullptr, stream);
 }
 
 extern "C" uint32_t s3r_tile_height(void) { return (uint32_t)TILE_H; }
@@ -1009,7 +1024,7 @@ static int render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint
                 }
                 return S3R_OK;
             };
-            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, ss_log2, r->frame.p, r->stream, bands, packed, copy_band);
+            int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, ss_log2, r->frame.p, nullptr, nullptr, r->stream, bands, packed, copy_band);
             if (rc) { return rc; }
             r->last_views = nv; r->last_W = W; r->last_H = H;
             // ---- drain: as each slice lands in staging the worker threads move it to the caller ----
@@ -1397,7 +1412,7 @@ int multi_worker_frame(MultiGpu *mg, int k) {
             if (tr && b < 16) { CUDA_TRY(cudaEventRecord(tr->ee[b], r->copy_stream)); }
             return S3R_OK;
         };
-        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, 0, r->frame.p, r->stream, mg->bands, false, copy_band);
+        int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, 0, r->frame.p, nullptr, nullptr, r->stream, mg->bands, false, copy_band);
         if (rc) { return rc; }
         r->last_views = 1; r->last_W = j.W; r->last_H = j.H; r->last_stream = r->stream;
         const auto t_launched = std::chrono::steady_clock::now();

@@ -73,7 +73,7 @@ EXPORTS = [
     "s3r_dropin_reset", "s3r_debug_walk", "s3r_debug_exact_math", "s3r_render_device_rows", "s3r_tile_height",
     "s3r_peer_frame_alloc", "s3r_peer_frame_open", "s3r_peer_frame_release", "s3r_set_peer_frames", "s3r_copy_from_device",
     "s3r_sink_open", "s3r_sink_submit", "s3r_sink_close", "s3r_debug_band_edges", "s3r_get_kernel_timing", "s3r_debug_clusters", "s3r_dropin_devices", "s3r_dropin_release_pins",
-    "s3r_render_device_ssaa", "s3r_render_host_ssaa",
+    "s3r_render_device_ssaa", "s3r_render_host_ssaa", "s3r_render_device_visibility",
 ]
 
 
@@ -129,6 +129,7 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.s3r_finish.argtypes = [vp]
     lib.s3r_render_host.argtypes = [vp, vp, u32, u32, u32, u32, u32, vp]
     lib.s3r_render_device_ssaa.argtypes = [vp, vp, u32, u32, u32, u32, u32, u32, vp, vp]
+    lib.s3r_render_device_visibility.argtypes = [vp, vp, u32, u32, u32, u32, u32, vp, vp, vp, vp]
     lib.s3r_render_host_ssaa.argtypes = [vp, vp, u32, u32, u32, u32, u32, u32, vp]
     lib.s3r_get_stats.argtypes = [vp, u32, ctypes.POINTER(CStats)]
     lib.s3r_dump_raster_vertices.argtypes = [vp, u32, vp, u64]
@@ -316,6 +317,18 @@ class Renderer:
         y1 = height if y1 is None else y1
         self._check(self._lib.s3r_render_device_ssaa(self._h, cams.ctypes.data, cams.shape[0], width, height, y0, y1,
                                                       samples, ctypes.c_void_p(dev_ptr), ctypes.c_void_p(stream)))
+
+    def render_device_visibility(self, cameras, width: int, height: int, colour_ptr: int = 0, triangle_ptr: int = 0,
+                                 depth_ptr: int = 0, y0: int = 0, y1: Optional[int] = None, stream: int = 0) -> None:
+        """``render_device`` that also writes the visibility planes, each laid out like the colour output in device
+        memory: per pixel the scene index of the winning triangle (uint32; a triangle the near-plane clip appended
+        reports its parent; background 0xFFFFFFFF) and its interpolated 1/z (float32; background +0).  A pointer of 0
+        leaves that output out; with ``colour_ptr`` = 0 nothing is shaded.  At least one pointer must be set."""
+        cams = np.ascontiguousarray(cameras, "<f4").reshape(-1, 12)
+        y1 = height if y1 is None else y1
+        self._check(self._lib.s3r_render_device_visibility(self._h, cams.ctypes.data, cams.shape[0], width, height, y0, y1,
+                                                            ctypes.c_void_p(colour_ptr), ctypes.c_void_p(triangle_ptr),
+                                                            ctypes.c_void_p(depth_ptr), ctypes.c_void_p(stream)))
 
     def render_device_rows(self, cameras, width: int, height: int, row_stride: int, row_phase: int, dev_ptr: int,
                            stream: int = 0) -> None:
