@@ -86,6 +86,40 @@ S3R_API int s3r_load_scene_arrays(S3RRenderer *r, const float *vertices_xyzw, ui
 S3R_API int s3r_scene_counts(const S3RRenderer *r, uint64_t *vertices, uint64_t *indices, uint64_t *attributes,
                      uint64_t *texels);
 
+/* ---- scene updates: new contents for the loaded scene, in place (animation) ---------------------
+ * Counts, both index streams and the number of atlases are fixed at load: an update overwrites contents and never
+ * reallocates the scene or the frame scratch (new geometry that needs more room takes the usual path: s3r_finish
+ * returns 1, render again).
+ *   s3r_update_vertices   positions of vertices [first, first + count): xyz holds count x 3 binary32, tightly packed
+ *                         (w stays 1; non-finite values are accepted, as at load).  source_on_device = 0: host memory,
+ *                         the call returns once the data has left the caller's buffer; 1: device memory of the renderer's
+ *                         device, read by the enqueued work — keep it unchanged until that work has run.  Every cluster
+ *                         of the load-time partition gets its private vertex copies gathered again and its bounds refit
+ *                         by the load-time rule (membership and order stay).  Enqueues 2 kernels (1 for a scene without
+ *                         triangles).
+ *   s3r_update_attributes records [first, first + count): 48-byte records as in data.bin, from host memory only,
+ *                         checked by the load rules (normal w == 0, kind <= 1, texture index < atlas count); a violation
+ *                         returns S3R_E_SCENE.  A copy, no kernel.
+ *   s3r_update_texels     atlases [first_atlas, first_atlas + atlases): atlases x 2^18 words, host or device memory
+ *                         (source_on_device as above; host data has left the caller's buffer on return).  A copy.
+ * Ordering: an update is enqueued on `stream` (a cudaStream_t, NULL = the renderer's own stream, the one s3r_render_host
+ * uses).  Work enqueued on that stream before the update renders the old scene, work enqueued after it the new one;
+ * across streams the caller orders, as for s3r_render_device.  s3r_dump_raster_vertices recomputes from the current
+ * positions on the cluster path, so after an update it may describe the updated scene.
+ * Errors (nothing is written): count = 0 is a no-op that enqueues nothing; a range past the scene, a null source with
+ * count > 0, a flag other than 0 / 1 or a source that is not where the flag says (cudaPointerGetAttributes; managed
+ * memory is neither) return S3R_E_ARG; no scene returns S3R_E_NOSCENE. */
+S3R_API int s3r_update_vertices(S3RRenderer *r, uint64_t first, uint64_t count, const float *xyz,
+                                int source_on_device, void *stream);
+S3R_API int s3r_update_attributes(S3RRenderer *r, uint64_t first, uint64_t count, const void *records_48b, void *stream);
+S3R_API int s3r_update_texels(S3RRenderer *r, uint32_t first_atlas, uint32_t atlases, const uint32_t *texels,
+                              int source_on_device, void *stream);
+/* Test hook: the device's cluster headers and cluster-private vertex copies as they are after all work enqueued so far,
+ * laid out like s3r_debug_clusters' outputs (hdr_out: clusters + 1 records of 32 bytes, pos_out: three planes of v_cap
+ * floats; each is filled when non-null and large enough).  counts_out = {clusters, cluster vertices, triangles}. */
+S3R_API int s3r_dump_clusters(S3RRenderer *r, void *hdr_out, uint64_t hdr_cap, float *pos_out, uint64_t v_cap,
+                              uint64_t counts_out[3]);
+
 /* ---- camera on the host (update_camera, render-cpp/render.cpp:134-156) --------------------- */
 S3R_API void s3r_camera_reset(S3RCamera *cam);
 S3R_API void s3r_camera_update(S3RCamera *cam, const S3RInput *input);

@@ -26,12 +26,6 @@ struct Raw {            // one finished cluster before sorting
     uint32_t morton;
 };
 
-inline float round_up(double v) {   // smallest-ish binary32 >= v, with one extra ulp of slack
-    float f = (float)v;
-    if (!(f >= v)) { f = nextafterf(f, INFINITY); }
-    return nextafterf(f, INFINITY);
-}
-
 inline uint32_t spread3(uint32_t v) {   // 10 bits -> every third bit
     v &= 1023u;
     v = (v | (v << 16)) & 0x030000FFu;
@@ -54,22 +48,11 @@ void build_clusters(const float *px, const float *py, const float *pz, const uin
         if (cur.n_tris == 0) { return; }
         Raw r;
         r.t0 = cur.t0; r.n_tris = cur.n_tris;
-        const float c[3] = {(float)(0.5 * (cur.lo[0] + cur.hi[0])), (float)(0.5 * (cur.lo[1] + cur.hi[1])), (float)(0.5 * (cur.lo[2] + cur.hi[2]))};
-        double r2 = 0;
-        for (uint32_t k = 0; k < cur.n_verts; k++) {
-            double d2 = 0;
-            for (int a = 0; a < 3; a++) { const double d = (double)pos[a][cur.verts[k]] - (double)c[a]; d2 += d * d; }
-            r2 = std::max(r2, d2);   // (a NaN never wins here; non-finite clusters are handled below)
-        }
-        r.cx = c[0]; r.cy = c[1]; r.cz = c[2];
-        r.radius = round_up(sqrt(r2) * (1.0 + 1e-9));
-        r.max_edge = round_up(sqrt(cur.max_edge2) * (1.0 + 1e-9));
-        bool finite = true;
-        for (uint32_t k = 0; k < cur.n_verts; k++) { for (int a = 0; a < 3; a++) { finite = finite && std::isfinite(pos[a][cur.verts[k]]); } }
-        if (!finite || !std::isfinite(r.radius) || !std::isfinite(r.max_edge)) {
-            // a vertex is NaN / infinite: bounds that can never justify a skip (every comparison against them fails)
-            r.cx = r.cy = r.cz = 0.f; r.radius = INFINITY; r.max_edge = INFINITY;
-        }
+        const ClusterBounds b = cluster_bounds(
+            cur.n_tris, cur.n_verts,
+            [&](uint32_t j, int c, int a) { return pos[a][(c == 0 ? vi0 : c == 1 ? vi1 : vi2)[cur.t0 + j]]; },
+            [&](uint32_t k, int a) { return pos[a][cur.verts[k]]; });
+        r.cx = b.cx; r.cy = b.cy; r.cz = b.cz; r.radius = b.radius; r.max_edge = b.max_edge;
         r.morton = 0;
         raw.push_back(r);
         cur.n_verts = 0; cur.n_tris = 0; cur.max_edge2 = 0;
@@ -143,8 +126,8 @@ void build_clusters(const float *px, const float *py, const float *pz, const uin
     out.n_clusters = (uint32_t)raw.size();
     out.hdr.resize(raw.size() + 1);
     out.tri.resize((size_t)T);
-    out.px.clear(); out.py.clear(); out.pz.clear();
-    out.px.reserve((size_t)T); out.py.reserve((size_t)T); out.pz.reserve((size_t)T);
+    out.px.clear(); out.py.clear(); out.pz.clear(); out.src.clear();
+    out.px.reserve((size_t)T); out.py.reserve((size_t)T); out.pz.reserve((size_t)T); out.src.reserve((size_t)T);
     uint32_t tri_off = 0;
     for (size_t k = 0; k < order.size(); k++) {
         const Raw &r = raw[order[k]];
@@ -162,6 +145,7 @@ void build_clusters(const float *px, const float *py, const float *pz, const uin
                 if (at == n_verts) {
                     verts[n_verts++] = id[c];
                     out.px.push_back(px[id[c]]); out.py.push_back(py[id[c]]); out.pz.push_back(pz[id[c]]);
+                    out.src.push_back(id[c]);
                 }
                 local[c] = at;
             }

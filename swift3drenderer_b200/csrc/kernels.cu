@@ -2343,6 +2343,38 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_CTAS) shade_tiles(const _
 }
 
 // ------------------------------------------------------------------------------------------------
+// scene updates (s3r_update_vertices): new positions in place, then every cluster refit
+// ------------------------------------------------------------------------------------------------
+// count x 3 packed binary32 (host-mapped staging or caller device memory) -> pos_x/y/z[first .. first + count)
+__global__ void __launch_bounds__(256) scene_scatter(const SceneUpdate u, const float *xyz, uint32_t first, uint32_t count) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) { return; }
+    const float x = xyz[3ull * i], y = xyz[3ull * i + 1], z = xyz[3ull * i + 2];
+    u.pos_x[first + i] = x; u.pos_y[first + i] = y; u.pos_z[first + i] = z;
+}
+
+// One thread per cluster, membership as built at load: the private copies are gathered again through cl_src, and the
+// bounds are recomputed from them by cluster_bounds (cluster.hpp), the rule build_clusters applies — same bits.  t0, v_off,
+// tri_off and the sentinel stay.
+__global__ void __launch_bounds__(256) cluster_refit(const SceneUpdate u) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= u.n_clusters) { return; }
+    const uint4 h = u.cl_hdr[2 * k + 1], next = u.cl_hdr[2 * k + 3];   // {max_edge, t0, v_off, tri_off}
+    const uint32_t v_off = h.z, n_verts = next.z - h.z, tri_off = h.w, n_tris = next.w - h.w;
+    float *cp[3] = {u.cl_px + v_off, u.cl_py + v_off, u.cl_pz + v_off};
+    for (uint32_t j = 0; j < n_verts; j++) {
+        const uint32_t s = u.cl_src[v_off + j];
+        cp[0][j] = u.pos_x[s]; cp[1][j] = u.pos_y[s]; cp[2][j] = u.pos_z[s];
+    }
+    const uint32_t *tri = u.cl_tri + tri_off;
+    const ClusterBounds b = cluster_bounds(
+        n_tris, n_verts, [&](uint32_t j, int c, int a) { return cp[a][(tri[j] >> (8 * c)) & 255u]; },
+        [&](uint32_t j, int a) { return cp[a][j]; });
+    u.cl_hdr[2 * k] = make_uint4(__float_as_uint(b.cx), __float_as_uint(b.cy), __float_as_uint(b.cz), __float_as_uint(b.radius));
+    reinterpret_cast<uint32_t *>(u.cl_hdr + 2 * k + 1)[0] = __float_as_uint(b.max_edge);
+}
+
+// ------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------
 static int g_sm_count = 148;
@@ -2458,6 +2490,19 @@ int launch_geometry_small(const Frame &f, cudaStream_t s, const LaunchMarks *m) 
     geometry_small<<<f.n_views, 256, 0, s>>>(f); mark(m, "geometry_small");
     if (!f.coltab) { return 1; }
     span_walk<<<dim3(ceil_div(f.H, 128u), SPAN_MAX * 3u, f.n_views), 128, 0, s>>>(f); mark(m, "span_walk");
+    return 2;
+}
+
+// Scene update: scatter, then (when the scene has clusters) the refit.  Both are plain launches, never chained, and trigger
+// no dependents: a plain launch starts only after the stream's previous kernel has completed and flushed, so the last
+// kernel of the render before (shade_tiles reads the raw scene for record-free triangles; the cluster front reads the
+// copies and headers) is done before a position changes.  The next render's first kernel (cluster_cull, vertex_stage or
+// geometry_small) is itself a plain launch, so it starts after the refit has completed and sees every write; the render's
+// chained kernels follow that one.
+int launch_scene_update(const SceneUpdate &u, const float *xyz, uint32_t first, uint32_t count, cudaStream_t s) {
+    scene_scatter<<<ceil_div(count, 256u), 256, 0, s>>>(u, xyz, first, count);
+    if (u.n_clusters == 0) { return 1; }
+    cluster_refit<<<ceil_div(u.n_clusters, 256u), 256, 0, s>>>(u);
     return 2;
 }
 

@@ -2,7 +2,7 @@
 //
 // HBM layout (all arrays 256-byte aligned cudaMalloc blocks):
 //
-//   scene (immutable after load; converted once from data.bin's AoS records)
+//   scene (converted once from data.bin's AoS records; contents rewritten in place by the s3r_update_* calls, counts fixed)
 //     pos_x/pos_y/pos_z   float[Vpad]        planar positions, streamed as float4 by the vertex stage
 //     vi0/vi1/vi2         uint32[T]          planar vertex-index streams (corner 0/1/2 of triangle t)
 //     ai0/ai1/ai2         uint32[T]          planar attribute-index streams
@@ -191,6 +191,16 @@ struct Frame {
     float *depth_out;
 };
 
+// Scene update (s3r_update_vertices): where new positions go and the cluster arrays the refit rewrites in place.
+struct SceneUpdate {
+    float *pos_x, *pos_y, *pos_z;
+    uint4 *cl_hdr;                // n_clusters + 1 headers (2 x uint4 each); the refit rewrites {cx, cy, cz, radius, max_edge}
+    float *cl_px, *cl_py, *cl_pz;
+    const uint32_t *cl_tri;
+    const uint32_t *cl_src;       // per cluster vertex: the original vertex index it copies
+    uint32_t n_clusters;
+};
+
 // Launchers (kernels.cu).  Each returns the number of kernels it enqueued.  `marks` (optional): called after every kernel
 // launch with the kernel's name — the host layer records a timing event there (option "timing").
 struct LaunchMarks { void (*fn)(void *ctx, const char *kernel); void *ctx; };
@@ -198,6 +208,8 @@ int launch_geometry(const Frame &f, cudaStream_t s, const LaunchMarks *marks = n
 int launch_raster(const Frame &f, cudaStream_t s, const LaunchMarks *marks = nullptr);     // per-tile visibility + shading + write-out
 int launch_geometry_small(const Frame &f, cudaStream_t s, const LaunchMarks *marks = nullptr);  // single-CTA-per-view fused geometry (+ span_walk when f.coltab is set)
 void launch_vertex_stage(const Frame &f, cudaStream_t s);   // vertex stage alone into f.rv (raster-vertex dumps)
+// positions xyz (count x 3 packed, device-readable) -> pos[first ..], then every cluster refit (plain launches)
+int launch_scene_update(const SceneUpdate &u, const float *xyz, uint32_t first, uint32_t count, cudaStream_t s);
 cudaError_t configure_kernels();
 void launch_exact_math(uint32_t mode, unsigned long long lo, unsigned long long count, uint32_t seed, unsigned long long *result,
                        cudaStream_t st);

@@ -142,7 +142,9 @@ struct S3RRenderer {
     DevBuf<uint4> cl_hdr;
     DevBuf<float> cl_px, cl_py, cl_pz;
     DevBuf<uint32_t> cl_tri;
+    DevBuf<uint32_t> cl_src;   // per cluster vertex: the original vertex it copies (scene updates re-gather the copies)
     uint32_t n_clusters = 0;
+    uint64_t n_cluster_verts = 0;
     int opt_clusters = 2, opt_cluster_cull = 1;   // clusters: 0 off, 1 on, 2 on for partitioned submissions
     Frame last_frame;   // parameter block of the last submission (raster-vertex dumps on the cluster path)
     FrameScratch scratch;
@@ -188,6 +190,11 @@ struct S3RRenderer {
     HostPins pins{cudaHostRegisterDefault};
     // fused frame assembly
     std::vector<void *> own_frames, opened_frames;
+    // scene updates from host memory: pinned, device-mapped staging; ev_update marks the end of the last update that read it
+    uint8_t *update_staging = nullptr;
+    size_t update_staging_bytes = 0;
+    cudaEvent_t ev_update = nullptr;
+    bool update_pending = false;
     uint32_t *peer_out[MAX_PEERS] = {};
     uint32_t n_peers = 0;
 };
@@ -207,6 +214,7 @@ static int create_device_objects(S3RRenderer *r) {
     CUDA_TRY(cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamCreateWithFlags(&r->aux_stream, cudaStreamNonBlocking));
     CUDA_TRY(cudaEventCreateWithFlags(&r->ev_geometry, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventCreateWithFlags(&r->ev_update, cudaEventDisableTiming));
     for (int i = 0; i < S3RRenderer::MAX_SLICES; i++) {
         CUDA_TRY(cudaEventCreateWithFlags(&r->ev_raster[i], cudaEventDisableTiming));
         CUDA_TRY(cudaEventCreateWithFlags(&r->ev_copy[i], cudaEventDisableTiming));
@@ -250,6 +258,8 @@ extern "C" void s3r_destroy(S3RRenderer *r) {
     delete r->copier;
     if (r->sticky_host) { cudaFreeHost(r->sticky_host); }
     if (r->staging) { cudaFreeHost(r->staging); }
+    if (r->update_staging) { cudaFreeHost(r->update_staging); }
+    if (r->ev_update) { cudaEventDestroy(r->ev_update); }
     for (int i = 0; i < S3RRenderer::MAX_SLICES; i++) {
         if (r->ev_raster[i]) { cudaEventDestroy(r->ev_raster[i]); cudaEventDestroy(r->ev_copy[i]); }
     }
@@ -267,6 +277,24 @@ extern "C" void s3r_destroy(S3RRenderer *r) {
 // --------------------------------------------------------------------------------------------------
 // scene: data.bin (render-cpp/render.cpp:177-209) -> HBM layout (pipeline.cuh)
 // --------------------------------------------------------------------------------------------------
+// 48-byte attribute records (data.bin) -> two uint4 each: {nx, ny, nz, kind}, {payload words 0..3}.  The load rules:
+// normal w == 0, kind <= 1, texture index < n_tex.  A violation returns S3R_E_SCENE; `out` may then be partly written.
+static int convert_attributes(const void *attributes, uint64_t A, uint32_t n_tex, uint4 *out) {
+    const uint8_t *rec = static_cast<const uint8_t *>(attributes);
+    for (uint64_t i = 0; i < A; i++) {
+        uint32_t w[12];
+        memcpy(w, rec + 48 * i, 48);
+        float nw;
+        memcpy(&nw, &w[3], 4);
+        if (nw != 0.0f) { return fail(S3R_E_SCENE, "normal w != 0"); }
+        if (w[8] > 1) { return fail(S3R_E_SCENE, "attribute kind not in {0, 1}"); }
+        if (w[8] == 1 && w[4] >= n_tex) { return fail(S3R_E_SCENE, "texture index out of range"); }
+        out[2 * i] = make_uint4(w[0], w[1], w[2], w[8]);
+        out[2 * i + 1] = make_uint4(w[4], w[5], w[6], w[7]);
+    }
+    return S3R_OK;
+}
+
 extern "C" int s3r_load_scene_arrays(S3RRenderer *r, const float *vertices, uint64_t V, const uint64_t *vidx,
                                      const uint64_t *aidx, uint64_t I, const void *attributes, uint64_t A,
                                      const uint32_t *texels, uint64_t n_texels) {
@@ -295,18 +323,8 @@ extern "C" int s3r_load_scene_arrays(S3RRenderer *r, const float *vertices, uint
     }
     const uint32_t n_tex = (uint32_t)(n_texels >> 18);
     std::vector<uint4> at(std::max<uint64_t>(2 * A, 2));
-    const uint8_t *rec = static_cast<const uint8_t *>(attributes);
-    for (uint64_t i = 0; i < A; i++) {
-        uint32_t w[12];
-        memcpy(w, rec + 48 * i, 48);
-        float nw;
-        memcpy(&nw, &w[3], 4);
-        if (nw != 0.0f) { return fail(S3R_E_SCENE, "normal w != 0"); }
-        if (w[8] > 1) { return fail(S3R_E_SCENE, "attribute kind not in {0, 1}"); }
-        if (w[8] == 1 && w[4] >= n_tex) { return fail(S3R_E_SCENE, "texture index out of range"); }
-        at[2 * i] = make_uint4(w[0], w[1], w[2], w[8]);
-        at[2 * i + 1] = make_uint4(w[4], w[5], w[6], w[7]);
-    }
+    const int arc = convert_attributes(attributes, A, n_tex, at.data());
+    if (arc) { return arc; }
     CUDA_TRY(r->pos_x.ensure(px.size())); CUDA_TRY(r->pos_y.ensure(px.size())); CUDA_TRY(r->pos_z.ensure(px.size()));
     CUDA_TRY(cudaMemcpy(r->pos_x.p, px.data(), px.size() * 4, cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(r->pos_y.p, py.data(), py.size() * 4, cudaMemcpyHostToDevice));
@@ -316,18 +334,20 @@ extern "C" int s3r_load_scene_arrays(S3RRenderer *r, const float *vertices, uint
         CUDA_TRY(cudaMemcpy(r->vi[k].p, v[k].data(), v[k].size() * 4, cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(r->ai[k].p, a[k].data(), a[k].size() * 4, cudaMemcpyHostToDevice));
     }
-    r->n_clusters = 0;
+    r->n_clusters = 0; r->n_cluster_verts = 0;
     if (T > 0) {   // clusters of consecutive, spatially close triangles for the general path's front kernel
         ClusterSet cs;
         build_clusters(px.data(), py.data(), pz.data(), v[0].data(), v[1].data(), v[2].data(), T, cs);
         CUDA_TRY(r->cl_hdr.ensure(cs.hdr.size() * 2)); CUDA_TRY(r->cl_px.ensure(cs.px.size())); CUDA_TRY(r->cl_py.ensure(cs.px.size()));
-        CUDA_TRY(r->cl_pz.ensure(cs.px.size())); CUDA_TRY(r->cl_tri.ensure(cs.tri.size()));
+        CUDA_TRY(r->cl_pz.ensure(cs.px.size())); CUDA_TRY(r->cl_tri.ensure(cs.tri.size())); CUDA_TRY(r->cl_src.ensure(cs.src.size()));
         CUDA_TRY(cudaMemcpy(r->cl_hdr.p, cs.hdr.data(), cs.hdr.size() * sizeof(ClusterHeader), cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(r->cl_px.p, cs.px.data(), cs.px.size() * 4, cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(r->cl_py.p, cs.py.data(), cs.py.size() * 4, cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(r->cl_pz.p, cs.pz.data(), cs.pz.size() * 4, cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(r->cl_tri.p, cs.tri.data(), cs.tri.size() * 4, cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(r->cl_src.p, cs.src.data(), cs.src.size() * 4, cudaMemcpyHostToDevice));
         r->n_clusters = cs.n_clusters;
+        r->n_cluster_verts = cs.px.size();
     }
     CUDA_TRY(r->attr.ensure(at.size()));
     CUDA_TRY(cudaMemcpy(r->attr.p, at.data(), at.size() * sizeof(uint4), cudaMemcpyHostToDevice));
@@ -423,6 +443,127 @@ extern "C" int s3r_debug_clusters(const float *vertices, uint64_t V, const uint6
 extern "C" int s3r_scene_counts(const S3RRenderer *r, uint64_t *v, uint64_t *i, uint64_t *a, uint64_t *t) {
     if (!r || !r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
     if (v) { *v = r->V; } if (i) { *i = r->I; } if (a) { *a = r->A; } if (t) { *t = r->n_texels; }
+    return S3R_OK;
+}
+
+// --------------------------------------------------------------------------------------------------
+// scene updates: new contents for a loaded scene, in place and ordered on a stream (include/s3r_b200.h)
+// --------------------------------------------------------------------------------------------------
+// The checks every update shares: renderer, scene, flag and range [first, first + count) within `total`.
+static int check_update(const S3RRenderer *r, uint64_t first, uint64_t count, uint64_t total, int source_on_device) {
+    if (!r) { return fail(S3R_E_ARG, "renderer is null"); }
+    if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
+    if (source_on_device != 0 && source_on_device != 1) { return fail(S3R_E_ARG, "source_on_device must be 0 or 1"); }
+    if (first > total || count > total - first) { return fail(S3R_E_ARG, "update range past the scene"); }
+    return S3R_OK;
+}
+
+// The source must be what the flag says: host memory (pageable or pinned) for 0, device memory of the renderer's device
+// for 1.
+static int check_source(const S3RRenderer *r, const void *src, int source_on_device) {
+    if (!src) { return fail(S3R_E_ARG, "source is null"); }
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, src) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
+    const bool on_device = at.type == cudaMemoryTypeDevice && at.device == r->device;
+    const bool on_host = at.type == cudaMemoryTypeUnregistered || at.type == cudaMemoryTypeHost;
+    if (source_on_device ? !on_device : !on_host) {
+        return fail(S3R_E_ARG, source_on_device ? "source is not device memory of the renderer's device" : "source is not host memory");
+    }
+    return S3R_OK;
+}
+
+// Pinned staging of at least `bytes` for a host-sourced update, once the previous update that read it has run.
+static int update_staging(S3RRenderer *r, size_t bytes, uint8_t **out) {
+    if (r->update_pending) { CUDA_TRY(cudaEventSynchronize(r->ev_update)); r->update_pending = false; }
+    if (bytes > r->update_staging_bytes) {
+        if (r->update_staging) { cudaFreeHost(r->update_staging); r->update_staging = nullptr; r->update_staging_bytes = 0; }
+        CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&r->update_staging), bytes, cudaHostAllocMapped));
+        r->update_staging_bytes = bytes;
+    }
+    *out = r->update_staging;
+    return S3R_OK;
+}
+
+static int staging_read_enqueued(S3RRenderer *r, cudaStream_t s) {
+    CUDA_TRY(cudaEventRecord(r->ev_update, s));
+    r->update_pending = true;
+    return S3R_OK;
+}
+
+extern "C" int s3r_update_vertices(S3RRenderer *r, uint64_t first, uint64_t count, const float *xyz, int source_on_device,
+                                   void *stream) {
+    int rc = check_update(r, first, count, r ? r->V : 0, source_on_device);
+    if (rc || count == 0) { return rc; }
+    CUDA_TRY(cudaSetDevice(r->device));
+    if ((rc = check_source(r, xyz, source_on_device))) { return rc; }
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
+    const float *src = xyz;
+    if (!source_on_device) {   // the caller's buffer is free when this returns; the scatter kernel reads the mapped staging
+        uint8_t *st = nullptr;
+        if ((rc = update_staging(r, (size_t)count * 12, &st))) { return rc; }
+        memcpy(st, xyz, (size_t)count * 12);
+        src = reinterpret_cast<const float *>(st);
+    }
+    SceneUpdate u;
+    u.pos_x = r->pos_x.p; u.pos_y = r->pos_y.p; u.pos_z = r->pos_z.p;
+    u.cl_hdr = r->cl_hdr.p; u.cl_px = r->cl_px.p; u.cl_py = r->cl_py.p; u.cl_pz = r->cl_pz.p;
+    u.cl_tri = r->cl_tri.p; u.cl_src = r->cl_src.p; u.n_clusters = r->n_clusters;
+    r->launches += (uint64_t)launch_scene_update(u, src, (uint32_t)first, (uint32_t)count, s);
+    CUDA_TRY(cudaGetLastError());
+    return source_on_device ? S3R_OK : staging_read_enqueued(r, s);
+}
+
+extern "C" int s3r_update_attributes(S3RRenderer *r, uint64_t first, uint64_t count, const void *records_48b, void *stream) {
+    int rc = check_update(r, first, count, r ? r->A : 0, 0);
+    if (rc || count == 0) { return rc; }
+    CUDA_TRY(cudaSetDevice(r->device));
+    if ((rc = check_source(r, records_48b, 0))) { return rc; }
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
+    uint8_t *st = nullptr;
+    if ((rc = update_staging(r, (size_t)count * 2 * sizeof(uint4), &st))) { return rc; }
+    if ((rc = convert_attributes(records_48b, count, (uint32_t)(r->n_texels >> 18), reinterpret_cast<uint4 *>(st)))) { return rc; }
+    CUDA_TRY(cudaMemcpyAsync(r->attr.p + 2 * first, st, (size_t)count * 2 * sizeof(uint4), cudaMemcpyHostToDevice, s));
+    return staging_read_enqueued(r, s);
+}
+
+extern "C" int s3r_update_texels(S3RRenderer *r, uint32_t first_atlas, uint32_t atlases, const uint32_t *texels,
+                                 int source_on_device, void *stream) {
+    int rc = check_update(r, first_atlas, atlases, r ? r->n_texels >> 18 : 0, source_on_device);
+    if (rc || atlases == 0) { return rc; }
+    CUDA_TRY(cudaSetDevice(r->device));
+    if ((rc = check_source(r, texels, source_on_device))) { return rc; }
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
+    const size_t bytes = (size_t)atlases << 20;   // 2^18 words per atlas
+    uint32_t *dst = r->texels.p + ((size_t)first_atlas << 18);
+    if (source_on_device) {
+        CUDA_TRY(cudaMemcpyAsync(dst, texels, bytes, cudaMemcpyDeviceToDevice, s));
+        return S3R_OK;
+    }
+    uint8_t *st = nullptr;
+    if ((rc = update_staging(r, bytes, &st))) { return rc; }
+    memcpy(st, texels, bytes);
+    CUDA_TRY(cudaMemcpyAsync(dst, st, bytes, cudaMemcpyHostToDevice, s));
+    return staging_read_enqueued(r, s);
+}
+
+// Test hook: the device's cluster headers and copies, after all work enqueued so far on the device.
+extern "C" int s3r_dump_clusters(S3RRenderer *r, void *hdr_out, uint64_t hdr_cap, float *pos_out, uint64_t v_cap,
+                                 uint64_t counts_out[3]) {
+    if (!r || !counts_out) { return fail(S3R_E_ARG, "null argument"); }
+    if (!r->has_scene) { return fail(S3R_E_NOSCENE, "no scene loaded"); }
+    counts_out[0] = r->n_clusters; counts_out[1] = r->n_cluster_verts; counts_out[2] = r->T;
+    if (r->n_clusters == 0) { return S3R_OK; }
+    CUDA_TRY(cudaSetDevice(r->device));
+    CUDA_TRY(cudaDeviceSynchronize());
+    if (hdr_out && hdr_cap > r->n_clusters) {
+        CUDA_TRY(cudaMemcpy(hdr_out, r->cl_hdr.p, ((size_t)r->n_clusters + 1) * sizeof(ClusterHeader), cudaMemcpyDeviceToHost));
+    }
+    if (pos_out && v_cap >= r->n_cluster_verts) {
+        const size_t b = r->n_cluster_verts * sizeof(float);
+        CUDA_TRY(cudaMemcpy(pos_out, r->cl_px.p, b, cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(pos_out + v_cap, r->cl_py.p, b, cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(pos_out + 2 * v_cap, r->cl_pz.p, b, cudaMemcpyDeviceToHost));
+    }
     return S3R_OK;
 }
 

@@ -74,6 +74,7 @@ EXPORTS = [
     "s3r_peer_frame_alloc", "s3r_peer_frame_open", "s3r_peer_frame_release", "s3r_set_peer_frames", "s3r_copy_from_device",
     "s3r_sink_open", "s3r_sink_submit", "s3r_sink_close", "s3r_debug_band_edges", "s3r_get_kernel_timing", "s3r_debug_clusters", "s3r_dropin_devices", "s3r_dropin_release_pins",
     "s3r_render_device_ssaa", "s3r_render_host_ssaa", "s3r_render_device_visibility",
+    "s3r_update_vertices", "s3r_update_attributes", "s3r_update_texels", "s3r_dump_clusters",
 ]
 
 
@@ -153,6 +154,10 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.s3r_sink_close.argtypes = [vp, ctypes.POINTER(u64)]
     lib.s3r_debug_band_edges.argtypes = [u32, ctypes.c_int, ctypes.c_int, ctypes.POINTER(u32), ctypes.c_int]
     lib.s3r_debug_clusters.argtypes = [vp, u64, vp, u64, vp, u64, vp, u64, vp, ctypes.POINTER(u64)]
+    lib.s3r_update_vertices.argtypes = [vp, u64, u64, vp, ctypes.c_int, vp]
+    lib.s3r_update_attributes.argtypes = [vp, u64, u64, vp, vp]
+    lib.s3r_update_texels.argtypes = [vp, u32, u32, vp, ctypes.c_int, vp]
+    lib.s3r_dump_clusters.argtypes = [vp, vp, u64, vp, u64, ctypes.POINTER(u64)]
     lib.s3r_get_kernel_timing.argtypes = [vp, u32, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(u64)]
     if path is None:
         _lib = lib
@@ -272,6 +277,44 @@ class Renderer:
         self._check(self._lib.s3r_load_scene_arrays(
             self._h, v.ctypes.data, v.shape[0], vi.ctypes.data, ai.ctypes.data, vi.shape[0], at.ctypes.data,
             at.shape[0], tx.ctypes.data, tx.size))
+
+    # ---- scene updates (include/s3r_b200.h): contents change in place, counts stay ---------------------------------------
+    @staticmethod
+    def _source(data, dtype, width):
+        """(pointer, element count, on device, keep-alive) of a host array or a contiguous CUDA tensor."""
+        if hasattr(data, "data_ptr") and getattr(data, "is_cuda", False):
+            assert data.is_contiguous() and data.element_size() == np.dtype(dtype).itemsize
+            return data.data_ptr(), data.numel() // width, 1, data
+        a = np.ascontiguousarray(data, dtype)
+        return a.ctypes.data, a.size // width, 0, a
+
+    def update_vertices(self, xyz, first: int = 0, stream: int = 0) -> None:
+        """New positions for vertices ``first ..``: a numpy (n, 3) float32 array (host) or a contiguous CUDA float32
+        tensor of n x 3 values (device; it must stay unchanged until the enqueued update has run).  Ordered on ``stream``
+        (0 = the renderer's own stream); the load-time clusters are refit on the GPU."""
+        ptr, n, dev, _keep = self._source(xyz, "<f4", 3)
+        self._check(self._lib.s3r_update_vertices(self._h, first, n, ctypes.c_void_p(ptr), dev, ctypes.c_void_p(stream)))
+
+    def update_attributes(self, records, first: int = 0, stream: int = 0) -> None:
+        """New attribute records (``scene.ATTR_DTYPE``, host) for attributes ``first ..``, checked by the load rules."""
+        at = np.ascontiguousarray(records)
+        assert at.dtype.itemsize == 48
+        self._check(self._lib.s3r_update_attributes(self._h, first, at.shape[0], at.ctypes.data, ctypes.c_void_p(stream)))
+
+    def update_textures(self, atlases, first: int = 0, stream: int = 0) -> None:
+        """New 512 x 512 atlases (uint32 0x00RRGGBB rip-maps) from ``first`` on: an array or a contiguous CUDA tensor."""
+        ptr, n, dev, _keep = self._source(atlases, "<u4", 1 << 18)
+        self._check(self._lib.s3r_update_texels(self._h, first, n, ctypes.c_void_p(ptr), dev, ctypes.c_void_p(stream)))
+
+    def cluster_dump(self) -> dict:
+        """The device's cluster headers (``CLUSTER_HDR_DTYPE``, with the sentinel) and planar copies (3, cluster vertices)."""
+        counts = (ctypes.c_uint64 * 3)()
+        self._check(self._lib.s3r_dump_clusters(self._h, None, 0, None, 0, counts))
+        nc, nv = int(counts[0]), int(counts[1])
+        hdr = np.zeros(nc + 1, CLUSTER_HDR_DTYPE)
+        pos = np.zeros((3, max(nv, 1)), np.float32)
+        self._check(self._lib.s3r_dump_clusters(self._h, hdr.ctypes.data, nc + 1, pos.ctypes.data, max(nv, 1), counts))
+        return {"hdr": hdr, "pos": pos[:, :nv]}
 
     def set_option(self, name: str, value: int) -> None:
         self._check(self._lib.s3r_set_option(self._h, name.encode(), int(value)))
