@@ -204,8 +204,10 @@ S3R_API int s3r_render_host_ssaa(S3RRenderer *r, const float *cameras, uint32_t 
                                  uint32_t y0, uint32_t y1, uint32_t samples_per_axis, uint32_t *host_out);
 
 /* ---- introspection (tests, bench) -------------------------------------------------------- */
+/* statistics of view `view` (its index in the last call's batch, whatever views_per_chunk split it into) */
 S3R_API int s3r_get_stats(S3RRenderer *r, uint32_t view, S3RStats *out);
-/* raster-space vertices of the last render of `view` (V x 4 floats: x, y, z, unused), render.cpp:285-289 */
+/* raster-space vertices of the last render of `view` (V x 4 floats: x, y, z, unused), render.cpp:285-289.  This and
+ * s3r_dump_setups keep only the views of the last chunk of a batch longer than views_per_chunk (S3R_E_ARG otherwise). */
 S3R_API int s3r_dump_raster_vertices(S3RRenderer *r, uint32_t view, float *out_xyzw, uint64_t capacity_vertices);
 /* surviving triangles of the last render of `view`, sorted by order key; *count receives the total */
 S3R_API int s3r_dump_setups(S3RRenderer *r, uint32_t view, S3RSetupDump *out, uint64_t capacity, uint64_t *count);

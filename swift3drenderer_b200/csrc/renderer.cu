@@ -175,6 +175,11 @@ struct S3RRenderer {
     uint64_t timed_chunks = 0;
     // last render (for finish / dumps)
     uint32_t last_views = 0, last_W = 0, last_H = 0;
+    // a batch longer than views_per_chunk: the per-view counters of every chunk but the last, copied out of the frame
+    // scratch (which the next chunk reuses) after each chunk; last_first = batch index of the last chunk's first view,
+    // last_total = views of the last call
+    DevBuf<uint32_t> batch_counters;
+    uint32_t last_first = 0, last_total = 0;
     cudaStream_t last_stream = nullptr;   // stream of the last s3r_render_device submission
     uint64_t launches = 0;
     int opt_tma = 1, opt_pin_host = 0;   // pinning caller memory is opt-in: see s3r_render_host
@@ -993,13 +998,18 @@ static int render_device(S3RRenderer *r, const float *cams, uint32_t n_views, ui
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : r->stream;
     r->last_stream = s;
     const size_t view_px = ((size_t)W * (row_stride == 1 ? y1 - y0 : (tile_rows - row_phase + row_stride - 1) / row_stride * TILE_H)) >> (2u * ss_log2);
+    if (n_views > r->views_per_chunk) { CUDA_TRY(r->batch_counters.ensure((size_t)n_views * C_COUNT)); }
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
         const size_t at = view_px * v0;   // (an output not requested stays null)
         int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, row_stride, row_phase, ss_log2, dev_out ? dev_out + at : dev_out,
                               dev_tri ? dev_tri + at : dev_tri, dev_depth ? dev_depth + at : dev_depth, s);
         if (rc) { return rc; }
-        r->last_views = nv;
+        if (v0 + nv < n_views) {
+            CUDA_TRY(cudaMemcpyAsync(r->batch_counters.p + (size_t)v0 * C_COUNT, r->scratch.counters.p, (size_t)nv * C_COUNT * sizeof(uint32_t),
+                                     cudaMemcpyDeviceToDevice, s));
+        }
+        r->last_views = nv; r->last_first = v0; r->last_total = n_views;
     }
     r->last_W = W; r->last_H = H;
     return S3R_OK;
@@ -1127,6 +1137,7 @@ static int render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint
     // main.swift:156-165).  A registration that outlives its memory poisons every later CUDA call that
     // touches a host pointer in the recycled range, so it is never done behind the caller's back.
     const bool pinned = r->opt_pin_host && r->pins.pin(host_out, view_px * n_views * 4);
+    if (n_views > r->views_per_chunk) { CUDA_TRY(r->batch_counters.ensure((size_t)n_views * C_COUNT)); }
     for (uint32_t v0 = 0; v0 < n_views; v0 += r->views_per_chunk) {
         const uint32_t nv = std::min(r->views_per_chunk, n_views - v0);
         uint32_t *dst = host_out + view_px * v0;
@@ -1167,7 +1178,7 @@ static int render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint
             };
             int rc = render_chunk(r, cams + 12 * (size_t)v0, nv, W, H, y0, y1, 1, 0, ss_log2, r->frame.p, nullptr, nullptr, r->stream, bands, packed, copy_band);
             if (rc) { return rc; }
-            r->last_views = nv; r->last_W = W; r->last_H = H;
+            r->last_views = nv; r->last_first = v0; r->last_total = n_views; r->last_W = W; r->last_H = H;
             // ---- drain: as each slice lands in staging the worker threads move it to the caller ----
             if (!pinned) { r->copier->begin(&slices, packed); }
             cudaError_t ce = cudaSuccess;
@@ -1190,6 +1201,10 @@ static int render_host(S3RRenderer *r, const float *cams, uint32_t n_views, uint
             }
         }
         if (!rendered) { return fail(S3R_E_CUDA, "frame scratch still overflowing after 8 regrowths"); }
+        if (v0 + nv < n_views) {
+            CUDA_TRY(cudaMemcpyAsync(r->batch_counters.p + (size_t)v0 * C_COUNT, r->scratch.counters.p, (size_t)nv * C_COUNT * sizeof(uint32_t),
+                                     cudaMemcpyDeviceToDevice, r->stream));
+        }
     }
     return S3R_OK;
 }
@@ -1277,10 +1292,12 @@ extern "C" int s3r_copy_from_device(S3RRenderer *r, void *host_dst, const void *
 // --------------------------------------------------------------------------------------------------
 extern "C" int s3r_get_stats(S3RRenderer *r, uint32_t view, S3RStats *out) {
     if (!r || !out) { return fail(S3R_E_ARG, "null argument"); }
-    if (view >= r->last_views) { return fail(S3R_E_ARG, "view out of range"); }
+    if (view >= r->last_total) { return fail(S3R_E_ARG, "view out of range"); }
     CUDA_TRY(cudaSetDevice(r->device));
     uint32_t c[C_COUNT];
-    CUDA_TRY(cudaMemcpy(c, r->scratch.counters.p + (size_t)view * C_COUNT, sizeof(c), cudaMemcpyDeviceToHost));
+    const uint32_t *src = view >= r->last_first ? r->scratch.counters.p + (size_t)(view - r->last_first) * C_COUNT
+                                                : r->batch_counters.p + (size_t)view * C_COUNT;
+    CUDA_TRY(cudaMemcpy(c, src, sizeof(c), cudaMemcpyDeviceToHost));
     memset(out, 0, sizeof(*out));
     out->triangles_in = (uint32_t)r->T;
     out->near_rejected = c[C_NEAR]; out->clipped = c[C_CLIPPED]; out->spawned = c[C_SPAWNED]; out->culled = c[C_CULLED];
@@ -1290,7 +1307,8 @@ extern "C" int s3r_get_stats(S3RRenderer *r, uint32_t view, S3RStats *out) {
 
 extern "C" int s3r_dump_raster_vertices(S3RRenderer *r, uint32_t view, float *out, uint64_t cap) {
     if (!r || !out) { return fail(S3R_E_ARG, "null argument"); }
-    if (view >= r->last_views || cap < r->V) { return fail(S3R_E_ARG, "view/capacity out of range"); }
+    if (view < r->last_first || view >= r->last_total || cap < r->V) { return fail(S3R_E_ARG, "view/capacity out of range (only the last chunk's views)"); }
+    view -= r->last_first;
     CUDA_TRY(cudaSetDevice(r->device));
     if (!r->last_frame.rv) {
         // the frame went through the cluster front, which keeps raster-space vertices in shared memory: run the vertex
@@ -1309,7 +1327,8 @@ extern "C" int s3r_dump_raster_vertices(S3RRenderer *r, uint32_t view, float *ou
 
 extern "C" int s3r_dump_setups(S3RRenderer *r, uint32_t view, S3RSetupDump *out, uint64_t cap, uint64_t *count) {
     if (!r || !count) { return fail(S3R_E_ARG, "null argument"); }
-    if (view >= r->last_views) { return fail(S3R_E_ARG, "view out of range"); }
+    if (view < r->last_first || view >= r->last_total) { return fail(S3R_E_ARG, "view out of range (only the last chunk's views)"); }
+    view -= r->last_first;
     CUDA_TRY(cudaSetDevice(r->device));
     uint32_t n = 0;
     CUDA_TRY(cudaMemcpy(&n, r->scratch.counters.p + (size_t)view * C_COUNT + C_SETUPS, 4, cudaMemcpyDeviceToHost));
@@ -1555,7 +1574,7 @@ int multi_worker_frame(MultiGpu *mg, int k) {
         };
         int rc = render_chunk(r, j.matrix, 1, j.W, j.H, 0, j.H, n, (uint32_t)k, 0, r->frame.p, nullptr, nullptr, r->stream, mg->bands, false, copy_band);
         if (rc) { return rc; }
-        r->last_views = 1; r->last_W = j.W; r->last_H = j.H; r->last_stream = r->stream;
+        r->last_views = 1; r->last_first = 0; r->last_total = 1; r->last_W = j.W; r->last_H = j.H; r->last_stream = r->stream;
         const auto t_launched = std::chrono::steady_clock::now();
         CUDA_TRY(cudaStreamSynchronize(r->copy_stream));
         const auto t_copied = std::chrono::steady_clock::now();

@@ -129,6 +129,44 @@ def test_batched_views_equal_single_views(gpu_renderer, renderer_lib):
     gpu_renderer.set_option("views_per_chunk", 256)
 
 
+def test_batch_statistics_name_the_batch_view_across_chunks(renderer_lib, oracle_port):
+    """stats(k) after a batch that views_per_chunk splits into chunks describes view k of the batch, on the host and the
+    device path and on both scene paths; the setup dump keeps the last chunk's views under their batch index.  (The
+    statistics were once read from the frame scratch, which holds only the last chunk: stats(0) of a batch of 7 in
+    chunks of 4 reported view 4, and stats(4) was refused.)"""
+    import torch
+    W, H = 160, 90
+    mats = renderer_lib.camera_path(S.input_script("spin", 12))[[3, 5, 6, 8, 9, 10, 11]]
+    for sc in (S.clip_stress_scene(60), S.clip_stress_scene(600)):   # 1 200 triangles (small-scene path), 12 000
+        osc = oracle_port.OracleScene(sc)
+        want = [osc.render(m, W, H, want_setups=True) for m in mats]
+        assert len({(o["stats"]["near_rejected"], o["stats"]["rasterized"]) for o in want}) == len(mats)
+        r = renderer_lib.Renderer(0)
+        try:
+            r.load_scene(sc)
+            r.set_option("views_per_chunk", 4)
+            r.set_option("direct_small", 0)
+            out = torch.zeros((len(mats), H, W), dtype=torch.int32, device="cuda:0")
+            for name, call in (("host", lambda: r.render(mats, W, H)),
+                               ("device", lambda: r.render_device(mats, W, H, out.data_ptr()))):
+                call()
+                assert r.finish() is False
+                for k, o in enumerate(want):
+                    st = r.stats(k)
+                    got = (st["near_rejected"], st["clipped"], st["spawned"], st["setups"], st["culled"])
+                    ref = (o["stats"]["near_rejected"], o["stats"]["clipped"], o["stats"]["spawned"], o["stats"]["rasterized"],
+                           o["stats"]["offscreen"] + o["stats"]["small_or_backfacing"])
+                    assert got == ref, f"T={sc.n_triangles} {name}: view {k} statistics {got} != oracle {ref}"
+                with pytest.raises(renderer_lib.RendererError):
+                    r.stats(len(mats))
+                for k in (4, 6):
+                    assert np.array_equal(r.setups(k)["order"], want[k]["setups"]["order"]), f"{name}: setups of view {k}"
+                with pytest.raises(renderer_lib.RendererError):
+                    r.setups(3)   # (an earlier chunk's records are gone)
+        finally:
+            r.close()
+
+
 def test_tma_and_plain_write_out_agree(gpu_renderer, renderer_lib):
     """tile_raster's three write-outs — one TMA tensor store per tile, bulk row copies, plain stores — on the host path
     (24-bit packed transport, banded launches) and the device path (32-bit, whole frame and a band that cuts tile rows),
